@@ -14,6 +14,9 @@ IHT iterations per second = (iterations summed over the K timed fits) / (device 
 `--impl reference` times that CPU restatement as the reference arm (Julia is not installed in this image).
 At N>1 the SNP columns are sharded over the ranks (weak scaling: p = 500,000 columns per GPU); at N=8 the line also
 carries `north_star`: BASELINE configs[4] (n=500k x p=1M, Normal, k=100, 10 covariates) strong-sharded over the 8 GPUs.
+`--dump-outputs DIR` writes the model of the last timed `value` fit (`--impl reference`: of its one fit) to
+DIR/<name>.npy in float64: the inputs are seeded, so two builds run with the same arguments can be compared output for
+output.
 """
 import argparse
 import json
@@ -40,10 +43,26 @@ PARITY_RTOL = 1e-6
 # One unit of work = one IHT iteration over one 50k x 500k shard.  At N=1 that is an IHT iteration of configs[1]; at N>1
 # (weak scaling, one shard per GPU) the job performs N shard-iterations per global iteration.
 UNIT = "iterations/s (x 500k-SNP shards)"
+DUMP_BYTES = 64 << 20
 
 
 def sweep_bytes(n, p):
     return p * ((n + 3) // 4) + 8 * n + 24 * p
+
+
+def dump_outputs(out_dir, res, beta, c):
+    """The model a caller of the timed fit receives: the dense beta, c, logl, iter and sigma_g, one float64 .npy each.
+    A beta larger than half of DUMP_BYTES (only at IHTB_BENCH_P sizes) is stored at a fixed, seeded sample of positions
+    joined with its support; beta_index.npy holds those positions."""
+    beta = np.asarray(beta, dtype=np.float64)
+    out = {"beta": beta, "c": c, "logl": [res.logl], "iter": [res.iter], "sigma_g": [res.sigma_g]}
+    if beta.nbytes > DUMP_BYTES // 2:
+        idx = np.random.default_rng(SEED).choice(beta.size, DUMP_BYTES // 32, replace=False)
+        idx = np.union1d(idx, np.flatnonzero(beta))
+        out["beta"], out["beta_index"] = beta[idx], idx
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measured_peak():
@@ -154,8 +173,10 @@ def run_reference(args):
     if rank != 0:
         return
     # one whole-workload fit at N=1 (about 40 s on 16 cores); at N>1 a 500k-column sample of the N x 500k problem
-    v, threads, sample, ms, _ = cpu_port_fit(N_SAMPLES, P_PER_GPU * args.gpus, K_SPARSITY, steps=1, warmup=0)
+    v, threads, sample, ms, ref = cpu_port_fit(N_SAMPLES, P_PER_GPU * args.gpus, K_SPARSITY, steps=1, warmup=0)
     assert threads > 1 or (os.cpu_count() or 1) == 1, "the CPU reference arm must use all host cores"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ref, ref.beta, ref.c)
     line = {
         "impl": "reference", "metric": "iht_iterations_per_sec", "value": v * args.gpus, "unit": UNIT,
         "global_iterations_per_sec": v,
@@ -234,6 +255,9 @@ def run_ours(args):
     m._lib.check(lib.ihtb_fit_phase_times(v._h, ph))
     phases = {k: ph[i] / max(iters + args.warmup * (iters // max(args.steps, 1)), 1) * 1e3
               for i, k in enumerate(["stepsize_ms", "gradstep_ms", "xb_glm_ms", "score_sweep_ms"])}
+    if args.dump_outputs:
+        beta_v, c_v, _, _ = v.get()
+        dump_outputs(args.dump_outputs, res, beta_v, c_v)
     v.close()
 
     # ---- e2e: public API, host buffers in / out every step ----
@@ -322,7 +346,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the model of the last timed fit to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -278,6 +278,8 @@ def bench_sharded(args, rank, world, local_rank, G):
     t_value = float(t.item()) * 1e-3
     beta, c, _, _ = v.get()
     v.close()
+    if rank == 0 and args.dump_outputs:
+        G["dump_outputs"](args.dump_outputs, res, beta, c)
 
     # e2e: public API with host y / z every step
     t0 = time.perf_counter()
