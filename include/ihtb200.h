@@ -46,7 +46,7 @@ enum { IHTB_LINK_IDENTITY = 0, IHTB_LINK_LOGIT = 1, IHTB_LINK_LOG = 2, IHTB_LINK
  *         re-score their candidates in FP64.  A single (or odd last) right-hand side takes the FAST path. */
 enum { IHTB_SWEEP_FAST = 0, IHTB_SWEEP_EXACT = 1, IHTB_SWEEP_PAIR = 2 };
 
-typedef struct ihtb_geno ihtb_geno;     /* replaces SnpLinAlg{Float64}(s; center, scale, impute) */
+typedef struct ihtb_geno ihtb_geno;     /* replaces SnpLinAlg{Float64}(s; center, scale, impute) or a dense Matrix{T} */
 typedef struct ihtb_fit ihtb_fit;       /* replaces IHTVariable{Float64, SnpLinAlg} (src/data_structures.jl:4-43) */
 typedef struct ihtb_mvfit ihtb_mvfit;   /* replaces mIHTVariable (src/data_structures.jl:140-180) */
 typedef struct ihtb_comm ihtb_comm;     /* NCCL communicator for SNP-sharded fits (no reference equivalent) */
@@ -146,6 +146,27 @@ int32_t ihtb_geno_ternary_tiles(const ihtb_geno* g, uint8_t* out, int64_t out_by
  * per-column decode kernel relative to the largest value. */
 int32_t ihtb_gather_bench(const ihtb_geno* g, int64_t ncols, int32_t reps, double* ms_per_call, double* max_rel_diff);
 int32_t ihtb_geno_destroy(ihtb_geno* g);
+
+/* ---- dense design matrix (fit_iht(y, x::AbstractMatrix{T}, z), src/fit.jl:62; T = Float64 or Float32) -------------
+ * The same ihtb_geno handle, holding an n x p matrix of real entries instead of 2-bit genotypes: imputed dosages from
+ * VCF / BGEN (src/wrapper.jl:406-423, 451-485) or any dense predictors.  Every univariate fit / CV / debias entry point
+ * takes it.  x: n x p column-major, column j at x + j*ld elements (ld >= n), element type dtype (stored on the device in
+ * that type; every kernel promotes entries exactly to FP64 and computes in FP64).
+ * standardize = 0: the matrix is used as given; a non-finite entry fails with IHTB_EDOMAIN at finalize.
+ * standardize = 1: standardize_genotypes! on the device: NaN = missing, mu_j = mean of the observed entries (fixed-order
+ *   sum), sigma_j = sqrt(mu_j (1 - mu_j/2)), missing -> mu_j, x = (g - mu_j) * (1/sigma_j) (1/sigma_j = 1 if sigma_j = 0):
+ *   integer dosages give the bits of ihtb_geno_decode of the same genotypes in a PLINK handle.
+ * On a DENSE handle ihtb_geno_stats returns the mu / sigma_inv / missing counts applied (0 / 1 / 0 with standardize = 0),
+ * ihtb_geno_decode the stored values, ihtb_geno_sweep_stream_bytes n*p*sizeof(T) with ternary = 0; ihtb_geno_packed,
+ * counts, maf, ternary_tiles, gather_bench and set_offset return IHTB_EUNSUPPORTED and load_columns IHTB_EINVAL.
+ * Not supported on a DENSE handle (IHTB_EUNSUPPORTED): multivariate fits, SNP-sharded fits, multi-device handles. */
+enum { IHTB_DENSE_F64 = 0, IHTB_DENSE_F32 = 1 };
+int32_t ihtb_geno_create_dense(const void* x, int32_t dtype, int64_t n, int64_t p, int64_t ld, int32_t standardize,
+                               ihtb_geno** out);
+/* piecewise form: create_dense_empty, load_dense_columns for columns [j_first, j_first+ncols) (any order, each column
+ * once; x + c*ld is column j_first + c), then ihtb_geno_finalize */
+int32_t ihtb_geno_create_dense_empty(int64_t n, int64_t p, int32_t dtype, int32_t standardize, ihtb_geno** out);
+int32_t ihtb_geno_load_dense_columns(ihtb_geno* g, const void* x, int64_t ld, int64_t j_first, int64_t ncols);
 
 /* ---- univariate fit (fit_iht / fit_iht! / init_iht_indices!, src/fit.jl:60-207, src/utilities.jl:366-438) ---- */
 /* y[n]; z is n x q column-major with the intercept in column 0; zkeep[q] (0/1) or NULL for all kept. */

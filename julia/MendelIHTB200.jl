@@ -95,9 +95,43 @@ mutable struct B200MultiSnpLinAlg <: AbstractMatrix{Float64}
     end
 end
 Base.size(x::B200MultiSnpLinAlg) = (x.n, x.p)
-const AnyB200 = Union{B200SnpLinAlg,B200MultiSnpLinAlg}
+
+# ---- dense design matrix (include/ihtb200.h ihtb_geno_create_dense) ----------------------------------------------
+"""Device-resident dense predictors: `fit_iht(y, x::AbstractMatrix{T}, z)` (src/fit.jl:62) for T = Float64 / Float32,
+e.g. the dosages `convert_gt` / `convert_bgen_gt` produce (src/wrapper.jl:406-485).  `standardize = true` runs
+`standardize_genotypes!` on the device (NaN = missing).  Stored as T, computed on in Float64; univariate fits only."""
+mutable struct B200DenseLinAlg{T<:Union{Float32,Float64}} <: AbstractMatrix{T}
+    handle::Ptr{Cvoid}
+    n::Int
+    p::Int
+    function B200DenseLinAlg(x::Matrix{T}; standardize::Bool=false) where {T<:Union{Float32,Float64}}
+        n, p = size(x)
+        h = Ref{Ptr{Cvoid}}(C_NULL)
+        check(ccall((:ihtb_geno_create_dense, LIB), Int32,
+                    (Ptr{Cvoid}, Int32, Int64, Int64, Int64, Int32, Ref{Ptr{Cvoid}}),
+                    x, T === Float32 ? 1 : 0, n, p, n, standardize, h))
+        g = new{T}(h[], n, p)
+        finalizer(g -> ccall((:ihtb_geno_destroy, LIB), Int32, (Ptr{Cvoid},), g.handle), g)
+        return g
+    end
+end
+Base.size(x::B200DenseLinAlg) = (x.n, x.p)
+function Base.getindex(x::B200DenseLinAlg{T}, i::Int, j::Int) where {T}     # the stored value
+    out = Ref{Float64}(0.0)
+    check(ccall((:ihtb_geno_decode, LIB), Int32, (Ptr{Cvoid}, Int64, Int64, Int64, Int64, Ref{Float64}),
+                x.handle, i - 1, i, j - 1, j, out))
+    T(out[])
+end
+function LinearAlgebra.mul!(out::AbstractVecOrMat{Float64}, xt::Transpose{<:Any,<:B200DenseLinAlg},
+                            v::AbstractVecOrMat{Float64})
+    check(ccall((:ihtb_xt_v, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Float64}, Int32),
+                xt.parent.handle, v, size(v, 2), out, 1))
+    out
+end
+
+const AnyB200 = Union{B200SnpLinAlg,B200MultiSnpLinAlg,B200DenseLinAlg}
 # the single-device and the multi-device calls have the same argument lists (ihtb_fit_* / ihtb_mfit_*)
-fitsym(::B200SnpLinAlg, name::Symbol) = Symbol(:ihtb_fit_, name)
+fitsym(::Union{B200SnpLinAlg,B200DenseLinAlg}, name::Symbol) = Symbol(:ihtb_fit_, name)
 fitsym(::B200MultiSnpLinAlg, name::Symbol) = Symbol(:ihtb_mfit_, name)
 mvsym(::B200SnpLinAlg, name::Symbol) = Symbol(:ihtb_mvfit_, name)          # multivariate: ihtb_mvfit_* / ihtb_mmvfit_*
 mvsym(::B200MultiSnpLinAlg, name::Symbol) = Symbol(:ihtb_mmvfit_, name)
@@ -148,7 +182,7 @@ function attach_options(x::AnyB200, fh, p::Int, k::Union{Int,Vector{Int}}, J::In
         check(ccall((fitsym(x, :set_weights), LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}), fh, weight))
     end
 end
-function fit_init(x::B200SnpLinAlg, fh, mask, init_beta::Bool)
+function fit_init(x::Union{B200SnpLinAlg,B200DenseLinAlg}, fh, mask, init_beta::Bool)
     check(ccall((init_beta ? :ihtb_fit_init_beta : :ihtb_fit_init, LIB), Int32, (Ptr{Cvoid}, Ptr{UInt8}), fh, mask))
 end
 function fit_init(x::B200MultiSnpLinAlg, fh, mask, init_beta::Bool)
@@ -290,7 +324,8 @@ function cv_iht(y::AbstractVector{Float64}, x::AnyB200, z::AbstractVecOrMat{Floa
         end
         return MendelIHT.meanloss(mses, q, folds)
     end
-    x isa B200SnpLinAlg || throw(ArgumentError("group / init_beta cross-validation runs on a single-device operator"))
+    x isa Union{B200SnpLinAlg,B200DenseLinAlg} ||
+        throw(ArgumentError("group / init_beta cross-validation runs on a single-device operator"))
     fh = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:ihtb_fit_create, LIB), Int32,
                 (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{UInt8}, Ref{Cfg}, Ref{Ptr{Cvoid}}),

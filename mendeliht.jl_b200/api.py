@@ -2,6 +2,8 @@
 
 Same names, argument meaning and error behaviour as the reference (all paths under /root/reference):
   `B200SnpLinAlg`  <- `SnpLinAlg{Float64}(s; model=ADDITIVE_MODEL, center, scale, impute)`  src/wrapper.jl:68-69
+  `B200DenseLinAlg` <- a dense `x::AbstractMatrix{T}`, T = Float64 / Float32  src/fit.jl:62 (standardize_genotypes!,
+                       src/wrapper.jl:406-423, on the device when asked)
   `fit_iht`        <- src/fit.jl:60-118        `IHTResult` <- src/data_structures.jl:245-258
   `cv_iht`         <- src/cross_validation.jl:60-131
   `iht`            <- src/wrapper.jl:52-120    `cross_validate` <- src/wrapper.jl:301-349
@@ -175,6 +177,95 @@ class B200SnpLinAlg:
                                     cm.ctypes.data_as(C.POINTER(C.c_double)), m,
                                     out.ctypes.data_as(C.POINTER(C.c_double))))
         return out[:, 0].copy() if one else out
+
+    def close(self):
+        if getattr(self, "_h", None):
+            load().ihtb_geno_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class B200DenseLinAlg:
+    """Device-resident dense n x p design matrix (float64 or float32 entries, computed on in FP64): imputed dosages from
+    VCF / BGEN or any real predictors.  Works wherever a single-GPU `B200SnpLinAlg` does in `fit_iht`, `cv_iht`, `cv_run`
+    and `IHTVariable` (univariate traits)."""
+
+    # host memory of the column-block upload of a C-ordered array (one block at a time)
+    _BLOCK_BYTES = 64 << 20
+
+    def __init__(self, handle, n, p, dtype, standardize):
+        self._h = handle
+        self.n, self.p = int(n), int(p)
+        self.dtype = np.dtype(dtype)
+        self.standardize = bool(standardize)
+
+    @classmethod
+    def from_array(cls, x: np.ndarray, standardize: bool = False) -> "B200DenseLinAlg":
+        """x: float64 or float32 ndarray [n, p].  standardize=True applies `standardize_genotypes!` on the device (NaN =
+        missing, imputed with the column mean; x = (g - mu) / sqrt(mu (1 - mu/2))); otherwise x is used as given and must
+        be finite.  A Fortran-ordered array (or column-major view) is read in place; any other layout is uploaded in
+        column blocks, so host memory grows by one block rather than by a transposed copy."""
+        if not isinstance(x, np.ndarray):
+            raise TypeError("x must be a numpy ndarray")
+        if x.ndim != 2:
+            raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"x must be a matrix (ndim 2), got ndim {x.ndim}")
+        if x.dtype == np.float64:
+            code = _lib.DENSE_F64
+        elif x.dtype == np.float32:
+            code = _lib.DENSE_F32
+        else:
+            raise TypeError(f"x must be float64 or float32, got {x.dtype}")
+        n, p = x.shape
+        if n == 0 or p == 0:
+            raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"x must have n > 0 and p > 0, got {x.shape}")
+        es = x.itemsize
+        lib = load()
+        h = C.c_void_p()
+        s0, s1 = x.strides
+        if s0 == es and s1 > 0 and s1 % es == 0 and s1 // es >= n:
+            check(lib.ihtb_geno_create_dense(C.c_void_p(x.ctypes.data), code, n, p, s1 // es, int(bool(standardize)),
+                                             C.byref(h)))
+            return cls(h, n, p, x.dtype, standardize)
+        check(lib.ihtb_geno_create_dense_empty(n, p, code, int(bool(standardize)), C.byref(h)))
+        obj = cls(h, n, p, x.dtype, standardize)
+        cols = max(1, cls._BLOCK_BYTES // (n * es))
+        for j in range(0, p, cols):
+            blk = np.asfortranarray(x[:, j:j + cols])
+            check(lib.ihtb_geno_load_dense_columns(h, C.c_void_p(blk.ctypes.data), n, j, blk.shape[1]))
+        check(lib.ihtb_geno_finalize(h))
+        return obj
+
+    @property
+    def shape(self):
+        return (self.n, self.p)
+
+    def size(self, dim=None):
+        return self.shape if dim is None else self.shape[dim - 1]
+
+    def stats(self):
+        """(mu, sigma_inv, n_missing) that standardization applied; (0, 1, 0) for a matrix used as given."""
+        return B200SnpLinAlg.stats(self)
+
+    def decode(self, i0=0, i1=None, j0=0, j1=None) -> np.ndarray:
+        """x[i0:i1, j0:j1] as stored on the device, float64."""
+        return B200SnpLinAlg.decode(self, i0, i1, j0, j1)
+
+    def xt_v(self, v: np.ndarray, mode: int = _lib.SWEEP_FAST) -> np.ndarray:
+        """x' v in FP64 for v [n] or [n, m] (every mode computes the same product)."""
+        return B200SnpLinAlg.xt_v(self, v, mode)
+
+    def x_support(self, idx, coef) -> np.ndarray:
+        """x[:, idx] * coef for coef [k] or [k, m], columns added in the order given."""
+        return B200SnpLinAlg.x_support(self, idx, coef)
+
+    def sweep_stream_bytes(self):
+        """(bytes one X'v sweep reads from HBM = n p sizeof(T), False)"""
+        return B200SnpLinAlg.sweep_stream_bytes(self)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -599,11 +690,14 @@ def fit_iht(y, x: B200SnpLinAlg, z=None, k=10, d=NORMAL, l=None, zkeep=None, est
     if J < 0:
         raise AssertionError("Value of J (max number of groups) must be nonnegative!\n")
     if is_multivariate(y):      # d = MvNormal: Y is r x n, Z is q x n (src/fit.jl:66,125)
+        if isinstance(x, B200DenseLinAlg):
+            raise _lib.IHTBError(_lib.IHTB_EUNSUPPORTED, "multivariate (MvNormal) fits need a B200SnpLinAlg: dense "
+                                                         "matrices serve univariate traits only")
         if debias:
             raise _lib.IHTBError(_lib.IHTB_EUNSUPPORTED,
                                  "Currently the debiasing routine for multivariate IHT is broken, sorry!")
         return _fit_mv(y, x, z, k, zkeep, tol, max_iter, min_iter, max_step, sweep_mode, init_beta, comm, p_global)
-    if not x.center:
+    if isinstance(x, B200SnpLinAlg) and not x.center:      # the reference checks SnpLinAlg only (src/fit.jl:97-101)
         raise _lib.IHTBError(_lib.IHTB_EUNSUPPORTED, "x is not centered! Please construct SnpLinAlg{Float64}"
                                                      "(::SnpArray, center=true, scale=true)")
     if z is None:
@@ -630,6 +724,8 @@ def fit_iht(y, x: B200SnpLinAlg, z=None, k=10, d=NORMAL, l=None, zkeep=None, est
 def maf_weights(x: B200SnpLinAlg, max_weight: float = np.inf) -> np.ndarray:
     """`maf_weights(x; max_weight)` (src/utilities.jl:692-697): w_j = 1 / (2 sqrt(p_j (1 - p_j))) clamped to
     [1, max_weight], p_j the minor allele frequency."""
+    if isinstance(x, B200DenseLinAlg):
+        raise TypeError("maf_weights needs genotypes (a B200SnpLinAlg), like the reference's maf_weights(x::SnpArray)")
     p = x.maf()
     with np.errstate(divide="ignore"):
         w = 1.0 / (2.0 * np.sqrt(p * (1.0 - p)))

@@ -126,9 +126,39 @@ static inline void ensure_dynamic_smem(K kernel, int bytes) {
 }
 
 // ---- genotype handle -----------------------------------------------------------------------
+struct TopkFuse;
+// dense.cu (DENSE handles).  The dense X'v is the plain product sum_i x_ij v_i: no centring, the mean of v is not read.
+ihtb_geno* dense_new_handle(int64_t n, int64_t p, int dtype, int standardize);
+void dense_upload(ihtb_geno* g, const void* x, int64_t ld_host, int64_t j_dst, int64_t ncols);
+void dense_finalize(ihtb_geno* g);       // statistics / standardization, error-bound scale; IHTB_EDOMAIN on bad entries
+int64_t dense_stream_bytes(const ihtb_geno* g);
+void dense_decode_block(const ihtb_geno* g, int64_t i0, int64_t i1, int64_t j0, int64_t j1, double* d_out);
+void dense_xt_v(const ihtb_geno* g, const double* dV, int64_t m, double* dOut, cudaStream_t s, DBuf<double>* part,
+                const TopkFuse* tf);
+void dense_sweep_kernel_only(const ihtb_geno* g, const double* dV, DBuf<double>* part, cudaStream_t s);
+void dense_x_support(const ihtb_geno* g, const int64_t* d_idx, int64_t k, const double* d_coef, int64_t m,
+                     double* d_out, cudaStream_t s);
+void dense_xt_gather2(const ihtb_geno* g, const int64_t* d_cols_a, int64_t n_a, const int64_t* d_cols_b, int64_t n_b,
+                      const double* d_v, int64_t m, double* d_out, cudaStream_t s);
+// sum_i w_i x_ij, sum_i w_i x_ij^2, sum_i wy_i x_ij per column (init_beta), three p-vectors
+void dense_init_beta_moments(const ihtb_geno* g, const double* d_w, const double* d_wy, double* d_sx, double* d_sxx,
+                             double* d_sxy, cudaStream_t s);
+// out[c*n + i] = x[i, cols[c]] in FP64 (cols[c] < 0: zeros)
+void dense_decode_cols(const ihtb_geno* g, const int64_t* d_cols, int64_t k, double* d_out, cudaStream_t s);
+// per-column scale and coefficient of the error bound of a sweep whose candidates are re-scored exactly:
+// |df_j - exact_j| <= coef * scale_j * (sum|r| + |sum r|).  PLINK: the handle's sinv and the sweep mode's coefficient.
+const double* geno_bound_scale(const ihtb_geno* g);
+double geno_bound_coef(const ihtb_geno* g, double plink_coef);
+
 }  // namespace ihtb
 
+// A handle holds one of two matrix kinds.  PLINK: the 2-bit packed genotypes below.  DENSE: an n x p matrix of FP64 or
+// FP32 entries (dense.cu), column-major with a padded leading dimension; the fit, CV and debias code reads it through
+// the dispatch points that test `kind`.
+enum { GENO_PLINK = 0, GENO_DENSE = 1 };
+
 struct ihtb_geno {
+    int kind = 0;             // GENO_PLINK | GENO_DENSE
     int device = 0;
     int64_t n = 0;            // samples
     int64_t p = 0;            // local SNP columns
@@ -166,7 +196,15 @@ struct ihtb_geno {
     ihtb::DBuf<int32_t> miss_idx;   // sample indices
     int64_t total_missing = 0;
     bool ready = false;             // columns loaded and statistics computed (false between create_empty and finalize)
+    // ---- DENSE handles (dense.cu) ----
+    int dtype = 0;                  // IHTB_DENSE_F64 | IHTB_DENSE_F32
+    int standardize = 0;            // 1: standardize_genotypes! applied at finalize (NaN = missing)
+    int64_t ld = 0;                 // device leading dimension in elements: n rounded up to a whole number of sweep slabs
+    ihtb::DBuf<uint8_t> dense;      // p * ld elements, zero padded below row n
+    ihtb::DBuf<double> dscale;      // per-column error-bound scale max_i |x_ij| of the stored (standardized) matrix
+    double dcoef = 0.0;             // error-bound coefficient of the dense sweep + re-scoring (dense_bound_coef)
 };
+static inline bool geno_is_dense(const ihtb_geno* g) { return g->kind == GENO_DENSE; }
 
 static inline void geno_require_ready(const ihtb_geno* g) {
     IHTB_CHECK(g && g->ready, IHTB_EINVAL, "genotype handle is not finalized (ihtb_geno_finalize)");
@@ -238,5 +276,23 @@ void xt_gather(const ihtb_geno* g, const int64_t* d_cols_local, int64_t ncols, c
 // is kept for source compatibility and ignored
 void xt_gather2(const ihtb_geno* g, const int64_t* d_cols_a, int64_t n_a, const int64_t* d_cols_b, int64_t n_b,
                 const double* d_v, int64_t m, const double* d_vsum, double* d_out, cudaStream_t s, bool blocked = false);
+
+struct TopkFuse;
+// dense.cu (DENSE handles).  The dense X'v is the plain product sum_i x_ij v_i: no centring, d_vbar is not read.
+void dense_xt_v(const ihtb_geno* g, const double* dV, int64_t m, double* dOut, cudaStream_t s, void* scratch_any,
+                const TopkFuse* tf);
+void dense_x_support(const ihtb_geno* g, const int64_t* d_idx, int64_t k, const double* d_coef, int64_t m,
+                     double* d_out, cudaStream_t s);
+void dense_xt_gather2(const ihtb_geno* g, const int64_t* d_cols_a, int64_t n_a, const int64_t* d_cols_b, int64_t n_b,
+                      const double* d_v, int64_t m, double* d_out, cudaStream_t s);
+// Sum_i w_i x_ij, Sum_i w_i x_ij^2, Sum_i wy_i x_ij per column (init_beta), three p-vectors
+void dense_init_beta_moments(const ihtb_geno* g, const double* d_w, const double* d_wy, double* d_sx, double* d_sxx,
+                             double* d_sxy, cudaStream_t s, void* scratch_any);
+// out[c*n + i] = x[i, cols[c]] in FP64 (cols[c] < 0: zeros)
+void dense_decode_cols(const ihtb_geno* g, const int64_t* d_cols, int64_t k, double* d_out, cudaStream_t s);
+// per-column scale and coefficient of the error bound of a sweep whose candidates are re-scored exactly
+// (|df_j - exact_j| <= coef * scale_j * (sum|r| + |sum r|)); PLINK: the handle's sinv with the sweep mode's coefficient
+const double* geno_bound_scale(const ihtb_geno* g);
+double geno_bound_coef(const ihtb_geno* g, double plink_coef);
 
 }  // namespace ihtb

@@ -192,7 +192,8 @@ void debias_irls(const ihtb_geno* g, const double* d_y, int dist, int link, doub
     const int64_t n = g->n;
     const int kk = k + 1;
     ws.ensure(n, k);
-    IHTB_LAUNCH(k_decode_cols, (unsigned)ceil_div(n * k, 256), 256, 0, s, geno_view(g), g->center, d_cols, (int64_t)k, ws.xk.p);
+    if (geno_is_dense(g)) dense_decode_cols(g, d_cols, k, ws.xk.p, s);
+    else IHTB_LAUNCH(k_decode_cols, (unsigned)ceil_div(n * k, 256), 256, 0, s, geno_view(g), g->center, d_cols, (int64_t)k, ws.xk.p);
     // SNP-sharded fits: every rank decodes its own support columns (zeros elsewhere); one all-reduce of the n x k block
     // gives all ranks the same dense matrix, and the refit then runs replicated
     if (comm) comm_allreduce_sum_f64(comm, ws.xk.p, (size_t)(n * k), s);

@@ -334,7 +334,7 @@ struct ihtb_fit {
         glm_score(glm, s, d_vbar.p);                         // scal: sum r, sum |r|, df2[q]; d_vbar[0] = scal[0] / n
         IHTB_CUDA(cudaMemcpyAsync(h_scal.p, d_scal.p, (2 + q) * sizeof(double), cudaMemcpyDeviceToHost, s));
         IHTB_CUDA(cudaEventRecord(ev0, s));
-        sweep_coef = cfg.sweep_mode == IHTB_SWEEP_FAST ? kFastBound : kExactBound;
+        sweep_coef = geno_bound_coef(g, cfg.sweep_mode == IHTB_SWEEP_FAST ? kFastBound : kExactBound);
         const double t_sw = now();
         if (pairer && cfg.sweep_mode == IHTB_SWEEP_FAST) {
             IHTB_CHECK(!grouped() && !comm, IHTB_EUNSUPPORTED, "paired sweeps serve plain single-device fits only");
@@ -346,7 +346,7 @@ struct ihtb_fit {
         } else if (cfg.k > 0 && !(grouped() && !init_plain)) {
             // the epilogue also runs the first stage of the candidate selection (keys of |df| with this sweep's error bound,
             // first digit histogram); select_rescore continues with topk_candidates_absdf_finish
-            const TopkFuse tf = topk_absdf_fuse_begin(tk, g->sinv.p, d_scal.p, sweep_coef);
+            const TopkFuse tf = topk_absdf_fuse_begin(tk, geno_bound_scale(g), d_scal.p, sweep_coef);
             sweep_xt_v_with_means(g, d_r.p, d_vbar.p, 1, d_dfa.p, cfg.sweep_mode, s, sweep_scratch, nullptr, nullptr, &tf);
         } else {
             sweep_xt_v_with_means(g, d_r.p, d_vbar.p, 1, d_dfa.p, cfg.sweep_mode, s, sweep_scratch, nullptr);
@@ -390,7 +390,7 @@ struct ihtb_fit {
             const bool paired = coef == kPairBound;        // L2 bound over the handle's sgn scale (see kPairBound)
             if (tk.fused_hist) topk_candidates_absdf_finish(tk, ksel, s);      // first stage done by the sweep epilogue
             else
-                topk_candidates_absdf(tk, d_dfa.p, paired ? g->sgn.p : g->sinv.p, rerun ? nullptr : d_scal.p, coef, ksel, s,
+                topk_candidates_absdf(tk, d_dfa.p, paired ? g->sgn.p : geno_bound_scale(g), rerun ? nullptr : d_scal.p, coef, ksel, s,
                                       bound, (paired && !rerun) ? pairer->d_l2 + pair_slot : nullptr);
             // slots re-scored without a second round trip; the looser bound of a PAIR sweep admits more near-threshold columns
             // (sized from the previous iteration's count there)
@@ -653,7 +653,7 @@ struct ihtb_fit {
         IHTB_CHECK(J >= 0, IHTB_EINVAL, "Value of J (max number of groups) must be nonnegative!");
         std::unique_ptr<GroupCtx> gc(new GroupCtx());
         std::vector<double> h_sinv((size_t)p);
-        IHTB_CUDA(cudaMemcpy(h_sinv.data(), g->sinv.p, (size_t)p * sizeof(double), cudaMemcpyDeviceToHost));
+        IHTB_CUDA(cudaMemcpy(h_sinv.data(), geno_bound_scale(g), (size_t)p * sizeof(double), cudaMemcpyDeviceToHost));
         gc->build(p, j0, p_global, group1, J, ks, n_groups, cfg.k, h_sinv.data());
         grpctx = std::move(gc);
     }
@@ -665,7 +665,7 @@ struct ihtb_fit {
         df_exact.clear(); cand_cache.clear();
         df_sparse = false; denom_ready = false;
         const double coef = sweep_coef;
-        group_topk(gc, d_dfa.p, g->sinv.p, rerun ? nullptr : d_scal.p, coef, bound, cfg.k, s);
+        group_topk(gc, d_dfa.p, geno_bound_scale(g), rerun ? nullptr : d_scal.p, coef, bound, cfg.k, s);
         const size_t G = (size_t)gc.G, nT = 2 * G + 1;
         const int nr = nranks();
         std::vector<double> TL(G), TU(G);
@@ -891,10 +891,16 @@ struct ihtb_fit {
         DBuf<double> cls((size_t)(7 * p));           // W1 W2 Wm Y1 Y2 Ym beta
         double *W1 = cls.p, *W2 = W1 + p, *Wm = W2 + p, *Y1 = Wm + p, *Y2 = Y1 + p, *Ym = Y2 + p, *bd = Ym + p;
         init_beta_products(glm, d_xs.p, s);                                   // d_xs = w .* y
-        sweep_class_sums(g, d_w.p, W1, W2, Wm, s, sweep_scratch);
-        sweep_class_sums(g, d_xs.p, Y1, Y2, Ym, s, sweep_scratch);
-        n_sweeps += 2;
-        init_beta_solve(glm, p, W1, W2, Wm, Y1, Y2, Ym, sum_w, sum_wy, g->mu.p, g->sinv.p, g->impute, bd, s);   // scal[0] = sum of intercepts
+        if (geno_is_dense(g)) {            // one pass: sum w x, sum w x^2, sum w y x of every column
+            dense_init_beta_moments(g, d_w.p, d_xs.p, W1, W2, Wm, s);
+            n_sweeps += 1;
+            init_beta_solve_moments(glm, p, W1, W2, Wm, sum_w, sum_wy, bd, s);
+        } else {
+            sweep_class_sums(g, d_w.p, W1, W2, Wm, s, sweep_scratch);
+            sweep_class_sums(g, d_xs.p, Y1, Y2, Ym, s, sweep_scratch);
+            n_sweeps += 2;
+            init_beta_solve(glm, p, W1, W2, Wm, Y1, Y2, Ym, sum_w, sum_wy, g->mu.p, g->sinv.p, g->impute, bd, s);
+        }                                                                     // scal[0] = sum of intercepts
         if (comm) comm_allreduce_sum_f64(comm, d_scal.p, 1, s);
         readback_scal(1);
         double c0sum = h_scal.p[0];
@@ -1433,6 +1439,8 @@ int32_t ihtb_fit_create_sharded(const ihtb_geno* g, ihtb_comm* comm, int64_t p_g
         IHTB_CHECK(g && y && z && cfg && out, IHTB_EINVAL, "NULL argument");
         IHTB_CHECK(p_global >= g->p, IHTB_EDIM, "p_global is smaller than the local shard");
         geno_require_ready(g);
+        IHTB_CHECK(!(geno_is_dense(g) && comm && comm->nranks > 1), IHTB_EUNSUPPORTED,
+                   "SNP-sharded fits need PLINK handles: a dense matrix is fitted on one device");
         IHTB_CHECK(q >= 1, IHTB_EDIM, "z must have at least the intercept column");
         IHTB_CHECK(cfg->k >= 0, IHTB_EINVAL, "Value of k (max predictors per group) must be nonnegative!");
         IHTB_CHECK(cfg->max_iter >= 0, IHTB_EINVAL, "Value of max_iter must be nonnegative!");

@@ -460,6 +460,7 @@ int32_t ihtb_geno_load_columns(ihtb_geno* g, const uint8_t* bed_cols, int64_t co
                                int64_t ncols) {
     return guard([&] {
         IHTB_CHECK(g && bed_cols, IHTB_EINVAL, "NULL argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EINVAL, "a dense handle takes ihtb_geno_load_dense_columns");
         IHTB_CHECK(!g->ready, IHTB_EINVAL, "genotype handle is already finalized");
         IHTB_CHECK(col_stride_bytes >= g->nbytes, IHTB_EDIM, "col_stride_bytes is smaller than ceil(n/4)");
         IHTB_CHECK(j_first >= 0 && ncols >= 0 && j_first + ncols <= g->p, IHTB_EDIM, "column range outside the matrix");
@@ -473,7 +474,12 @@ int32_t ihtb_geno_finalize(ihtb_geno* g) {
         IHTB_CHECK(g, IHTB_EINVAL, "NULL argument");
         IHTB_CHECK(!g->ready, IHTB_EINVAL, "genotype handle is already finalized");
         IHTB_CUDA(cudaSetDevice(g->device));
-        seal_handle(g);
+        if (geno_is_dense(g)) {
+            dense_finalize(g);
+            g->ready = true;
+        } else {
+            seal_handle(g);
+        }
     });
 }
 
@@ -534,6 +540,11 @@ int32_t ihtb_geno_sweep_stream_bytes(const ihtb_geno* g, int64_t* bytes, int32_t
     return guard([&] {
         IHTB_CHECK(g, IHTB_EINVAL, "NULL genotype handle");
         geno_require_ready(g);
+        if (geno_is_dense(g)) {
+            if (bytes) *bytes = dense_stream_bytes(g);
+            if (ternary) *ternary = 0;
+            return;
+        }
         const bool t = g->tern.p != nullptr;
         if (bytes) *bytes = (t ? g->tern_slabs : g->stride / 128) * g->p4 * 128;
         if (ternary) *ternary = t ? 1 : 0;
@@ -543,6 +554,7 @@ int32_t ihtb_geno_sweep_stream_bytes(const ihtb_geno* g, int64_t* bytes, int32_t
 int32_t ihtb_geno_set_offset(ihtb_geno* g, int64_t j0) {
     return guard([&] {
         IHTB_CHECK(g && j0 >= 0, IHTB_EINVAL, "bad argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "dense handles cannot be SNP shards");
         g->j0 = j0;
     });
 }
@@ -573,6 +585,7 @@ int32_t ihtb_geno_stats(const ihtb_geno* g, double* mu, double* sigma_inv, int64
 int32_t ihtb_geno_counts(const ihtb_geno* g, int64_t* counts) {
     return guard([&] {
         IHTB_CHECK(g && counts, IHTB_EINVAL, "NULL argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "genotype counts need a PLINK handle");
         geno_require_ready(g);
         IHTB_CUDA(cudaSetDevice(g->device));
         DBuf<int64_t> d((size_t)(4 * g->p));
@@ -584,6 +597,7 @@ int32_t ihtb_geno_counts(const ihtb_geno* g, int64_t* counts) {
 int32_t ihtb_geno_maf(const ihtb_geno* g, double* maf) {
     return guard([&] {
         IHTB_CHECK(g && maf, IHTB_EINVAL, "NULL argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "maf needs a PLINK handle (SnpArray)");
         geno_require_ready(g);
         IHTB_CUDA(cudaSetDevice(g->device));
         IHTB_CUDA(cudaMemcpy(maf, g->mu.p, g->p * sizeof(double), cudaMemcpyDeviceToHost));
@@ -604,7 +618,8 @@ int32_t ihtb_geno_decode(const ihtb_geno* g, int64_t i0, int64_t i1, int64_t j0,
         int64_t total = (i1 - i0) * (j1 - j0);
         if (total == 0) return;
         DBuf<double> d((size_t)total);
-        IHTB_LAUNCH(k_decode, (unsigned)ceil_div(total, 256), 256, 0, 0, geno_view(g), g->center, i0, i1, j0, j1, d.p);
+        if (geno_is_dense(g)) dense_decode_block(g, i0, i1, j0, j1, d.p);
+        else IHTB_LAUNCH(k_decode, (unsigned)ceil_div(total, 256), 256, 0, 0, geno_view(g), g->center, i0, i1, j0, j1, d.p);
         IHTB_CUDA(cudaMemcpy(out, d.p, total * sizeof(double), cudaMemcpyDeviceToHost));
     });
 }
@@ -612,6 +627,7 @@ int32_t ihtb_geno_decode(const ihtb_geno* g, int64_t i0, int64_t i1, int64_t j0,
 int32_t ihtb_geno_packed(const ihtb_geno* g, int64_t j0, int64_t j1, uint8_t* out) {
     return guard([&] {
         IHTB_CHECK(g && out, IHTB_EINVAL, "NULL argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "a dense handle has no packed genotypes");
         IHTB_CHECK(0 <= j0 && j0 <= j1 && j1 <= g->p, IHTB_EDIM, "column range out of bounds");
         geno_require_ready(g);
         IHTB_CUDA(cudaSetDevice(g->device));
@@ -633,6 +649,7 @@ int32_t ihtb_geno_packed(const ihtb_geno* g, int64_t j0, int64_t j1, uint8_t* ou
 int32_t ihtb_geno_ternary_tiles(const ihtb_geno* g, uint8_t* out, int64_t out_bytes) {
     return guard([&] {
         IHTB_CHECK(g && out, IHTB_EINVAL, "NULL argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "a dense handle has no ternary copy");
         geno_require_ready(g);
         IHTB_CHECK(g->tern.p != nullptr, IHTB_EINVAL, "this handle holds no ternary copy");
         const int64_t bytes = g->tern_slabs * g->p4 * 128;

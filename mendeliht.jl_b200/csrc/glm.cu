@@ -208,8 +208,21 @@ __global__ void k_wy(int64_t n, const double* __restrict__ w, const double* __re
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < n) out[i] = w[i] * y[i];
 }
-// per SNP: regression of y on [1, x_j] over the weighted samples from the class sums; slope clamped to [-2, 2];
-// a failed 2x2 Cholesky leaves (sum y, sum x y) like the reference's try/catch.  part[block] = sum of intercepts.
+// regression of y on [1, x_j] from N = sum w, SY = sum w y, sx, sxx, sxy by a 2x2 Cholesky; a failed factorisation
+// leaves (SY, sxy) like the reference's try/catch (src/utilities.jl:776-842); the slope is clamped to [-2, 2]
+__device__ __forceinline__ void init_beta_regress(double N, double SY, double sx, double sxx, double sxy, double& beta,
+                                                  double& icpt) {
+    double slope = sxy;
+    icpt = SY;
+    const double u11 = sqrt(N), u12 = sx / u11, dd = sxx - u12 * u12;
+    if (N > 0.0 && dd > 0.0) {
+        const double u22 = sqrt(dd), t1 = SY / u11, t2 = (sxy - u12 * t1) / u22;
+        slope = t2 / u22;
+        icpt = (t1 - u12 * slope) / u11;
+    }
+    beta = fmin(fmax(slope, -2.0), 2.0);
+}
+// per SNP: regression of y on [1, x_j] over the weighted samples from the class sums.  part[block] = sum of intercepts.
 __global__ void __launch_bounds__(GLM_THREADS)
 k_init_beta(int64_t p, const double* __restrict__ W1, const double* __restrict__ W2, const double* __restrict__ Wm,
             const double* __restrict__ Y1, const double* __restrict__ Y2, const double* __restrict__ Ym, double N,
@@ -225,14 +238,23 @@ k_init_beta(int64_t p, const double* __restrict__ W1, const double* __restrict__
         const double sx = a0 * w0 + a1 * w1 + a2 * w2 + am * wm;
         const double sxx = a0 * a0 * w0 + a1 * a1 * w1 + a2 * a2 * w2 + am * am * wm;
         const double sxy = a0 * y0 + a1 * y1 + a2 * y2 + am * ym;
-        double icpt = SY, slope = sxy;
-        const double u11 = sqrt(N), u12 = sx / u11, dd = sxx - u12 * u12;
-        if (N > 0.0 && dd > 0.0) {
-            const double u22 = sqrt(dd), t1 = SY / u11, t2 = (sxy - u12 * t1) / u22;
-            slope = t2 / u22;
-            icpt = (t1 - u12 * slope) / u11;
-        }
-        beta[j] = fmin(fmax(slope, -2.0), 2.0);
+        double icpt;
+        init_beta_regress(N, SY, sx, sxx, sxy, beta[j], icpt);
+        acc += icpt;
+    }
+    acc = block_sum(acc, sh);
+    if (threadIdx.x == 0) part[blockIdx.x] = acc;
+}
+// the same regressions from per-column moments (dense handles: sum w x, sum w x^2, sum w y x, dense.cu)
+__global__ void __launch_bounds__(GLM_THREADS)
+k_init_beta_moments(int64_t p, const double* __restrict__ SX, const double* __restrict__ SXX,
+                    const double* __restrict__ SXY, double N, double SY, double* __restrict__ beta,
+                    double* __restrict__ part) {
+    __shared__ double sh[32];
+    double acc = 0.0;
+    for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < p; j += (int64_t)gridDim.x * blockDim.x) {
+        double icpt;
+        init_beta_regress(N, SY, SX[j], SXX[j], SXY[j], beta[j], icpt);
         acc += icpt;
     }
     acc = block_sum(acc, sh);
@@ -268,6 +290,12 @@ void init_beta_solve(GlmCtx& c, int64_t p, const double* W1, const double* W2, c
                      int impute, double* d_beta, cudaStream_t s) {
     int grid = glm_grid(p);
     IHTB_LAUNCH(k_init_beta, grid, GLM_THREADS, 0, s, p, W1, W2, Wm, Y1, Y2, Ym, N, SY, mu, sinv, impute, d_beta, c.part);
+    IHTB_LAUNCH(k_finalize, 1, 32, 0, s, c.part, grid, 1, c.scal);
+}
+void init_beta_solve_moments(GlmCtx& c, int64_t p, const double* SX, const double* SXX, const double* SXY, double N,
+                             double SY, double* d_beta, cudaStream_t s) {
+    int grid = glm_grid(p);
+    IHTB_LAUNCH(k_init_beta_moments, grid, GLM_THREADS, 0, s, p, SX, SXX, SXY, N, SY, d_beta, c.part);
     IHTB_LAUNCH(k_finalize, 1, 32, 0, s, c.part, grid, 1, c.scal);
 }
 void init_beta_cov_sums(GlmCtx& c, cudaStream_t s) {

@@ -132,6 +132,9 @@ void init_beta_products(GlmCtx& c, double* d_wy, cudaStream_t s);             //
 void init_beta_solve(GlmCtx& c, int64_t p, const double* W1, const double* W2, const double* Wm, const double* Y1,
                      const double* Y2, const double* Ym, double N, double SY, const double* mu, const double* sinv,
                      int impute, double* d_beta, cudaStream_t s);                   // scal[0] = sum of intercepts
+// dense handles: the same regressions from per-column sums of w x, w x^2 and w y x
+void init_beta_solve_moments(GlmCtx& c, int64_t p, const double* SX, const double* SXX, const double* SXY, double N,
+                             double SY, double* d_beta, cudaStream_t s);
 void init_beta_cov_sums(GlmCtx& c, cudaStream_t s);                               // scal[3(l-1)+{0,1,2}]
 void glm_set_weights(GlmCtx& c, const uint8_t* d_mask, cudaStream_t s);        // scal: sum w, sum y*w
 

@@ -417,9 +417,9 @@ static int32_t cv_farm(const std::vector<ihtb_geno*>& parts, const std::vector<i
     const char* pe = getenv("IHTB_CV_PAIR");                  // read per call: tests switch it
     const int pair_env = pe ? atoi(pe) : -1;
     const bool want_pair = pair_env == 1 || (pair_env != 0 && n <= 131072);
-    // the pair sweep needs a tiled layout, FAST arithmetic and at least two fits to pair
+    // the pair sweep needs a tiled PLINK layout (a dense handle never pairs), FAST arithmetic and at least two fits
     const int per_dev = (want_pair && c.sweep_mode == IHTB_SWEEP_FAST && c.est_r == 0 && ngrid >= 2 &&
-                         parts[0]->cs_j == 128) ? 2 : 1;
+                         !geno_is_dense(parts[0]) && parts[0]->cs_j == 128) ? 2 : 1;
     std::vector<std::unique_ptr<SweepPairer>> pairers((size_t)nd);
     if (per_dev == 2) {
         rc = guard([&] { for (int d = 0; d < nd; ++d) pairers[(size_t)d].reset(new SweepPairer(devices[(size_t)d])); });

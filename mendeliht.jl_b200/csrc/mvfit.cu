@@ -822,6 +822,8 @@ int32_t ihtb_mvfit_create_sharded(const ihtb_geno* g, ihtb_comm* comm, int64_t p
     return guard([&] {
         IHTB_CHECK(g && Y && z && cfg && out, IHTB_EINVAL, "NULL argument");
         geno_require_ready(g);
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "multivariate (MvNormal) fits need a PLINK handle: dense matrices "
+                                                         "serve univariate fits only");
         IHTB_CHECK(p_global >= g->p, IHTB_EDIM, "p_global is smaller than the local shard");
         IHTB_CHECK(r >= 2 && r <= MV_MAXR, IHTB_EUNSUPPORTED, "multivariate IHT supports 2..20 traits");
         IHTB_CHECK(cfg->sweep_mode == IHTB_SWEEP_FAST || cfg->sweep_mode == IHTB_SWEEP_EXACT ||

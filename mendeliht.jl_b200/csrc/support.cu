@@ -107,6 +107,7 @@ void x_support_push(const ihtb_geno* g, const int64_t* d_idx, int64_t k, const d
 
 void x_support(const ihtb_geno* g, const int64_t* d_idx, int64_t k, const double* d_coef, int64_t m, double* d_out,
                cudaStream_t s) {
+    if (geno_is_dense(g)) { dense_x_support(g, d_idx, k, d_coef, m, d_out, s); return; }
     // m right-hand sides in groups of <= 4 (coef is k x m column-major, out is n x m column-major)
     for (int64_t t0 = 0; t0 < m;) {
         int64_t mm = m - t0;
@@ -307,6 +308,7 @@ void xt_gather2(const ihtb_geno* g, const int64_t* d_cols_a, int64_t n_a, const 
                 const double* d_v, int64_t m, const double* d_vbar, double* d_out, cudaStream_t s, bool blocked) {
     const int64_t ncols = n_a + n_b;
     if (ncols == 0) return;
+    if (geno_is_dense(g)) { dense_xt_gather2(g, d_cols_a, n_a, d_cols_b, n_b, d_v, m, d_out, s); return; }   // plain dots
     for (int64_t t0 = 0; t0 < m;) {
         int64_t mm = m - t0;
         const double* vv = d_v + t0 * g->n;
@@ -344,6 +346,7 @@ extern "C" int32_t ihtb_gather_bench(const ihtb_geno* g, int64_t ncols, int32_t 
                                      double* max_rel_diff) {
     return guard([&] {
         IHTB_CHECK(g && ncols >= 1 && reps >= 1, IHTB_EINVAL, "bad argument");
+        IHTB_CHECK(!geno_is_dense(g), IHTB_EUNSUPPORTED, "the gather bench times the PLINK re-scoring kernels");
         geno_require_ready(g);
         IHTB_CUDA(cudaSetDevice(g->device));
         cudaStream_t s;

@@ -207,49 +207,54 @@ void sweep_xt_v_with_means(const ihtb_geno* g, const double* dV, const double* d
         IHTB_CUDA(cudaEventCreate(&e0)); IHTB_CUDA(cudaEventCreate(&e1));
         IHTB_CUDA(cudaEventRecord(e0, s));
     }
-    if (d_l2)
-        for (int64_t t = 0; t < m; ++t) IHTB_LAUNCH(k_l2norm, 1, 1024, 0, s, dV + t * g->n, g->n, d_vbar + t, d_l2 + t);
-    for (int64_t t = 0; t < m; ++t) {
-        const double* v = dV + t * g->n;
-        double* out = dOut + t * g->p;
-        if (mode == IHTB_SWEEP_PAIR && g->cs_j == 128 && t + 1 < m) {
-            // two right-hand sides per pass over the matrix (half2 tables); an odd last one takes the FAST path below
-            const int64_t n_slabs = sweep_fast_num_slabs(g);
-            if (sc->part32.n < (size_t)(2 * n_slabs * g->p)) sc->part32.alloc((size_t)(2 * n_slabs * g->p));
-            if (sc->scale.n < 2) sc->scale.alloc(2);
-            IHTB_LAUNCH(k_pair_scale, 1, 1024, 0, s, v, v + g->n, g->n, d_vbar + t, sc->scale.p);
-            sweep_pair_partials(g, v, v + g->n, d_vbar + t, sc->scale.p, sc->part32.p, s);
-            for (int h = 0; h < 2; ++h)
-                IHTB_LAUNCH((k_sweep_epilogue<float>), (unsigned)ceil_div(g->p, 256), 256, 0, s,
-                            sc->part32.p + (size_t)h * n_slabs * g->p, n_slabs, g->p, g->mu.p, g->sinv.p, g->nmiss.p,
-                            g->miss_ptr.p, g->miss_idx.p, v + h * g->n, d_vbar + t + h, g->impute, out + h * g->p,
-                            sc->scale.p + h);
-            ++t;
-            continue;
-        }
-        if (mode == IHTB_SWEEP_EXACT && exact_uses_lut(g)) {
-            const int64_t n_slabs = g->stride / 128;
-            if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
-            sweep_exact_lut_partials(g, v, d_vbar + t, sc->part64.p, s);
-            IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
-                        g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
-                        g->impute, out, (const float*)nullptr, fuse);
-        } else if (mode == IHTB_SWEEP_EXACT) {
-            int64_t words = g->stride >> 2;
-            int64_t n_slabs = ceil_div(words, EX_THREADS);
-            if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
-            dim3 grid((unsigned)ceil_div(g->p, EX_COLS_PER_CTA), (unsigned)n_slabs);
-            IHTB_LAUNCH(k_sweep_exact, grid, EX_THREADS, 0, s, geno_view(g), v, d_vbar + t, sc->part64.p);
-            IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
-                        g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
-                        g->impute, out, (const float*)nullptr, fuse);
-        } else {
-            int64_t n_slabs = sweep_fast_num_slabs(g);
-            if (sc->part32.n < (size_t)(n_slabs * g->p)) sc->part32.alloc((size_t)(n_slabs * g->p));
-            sweep_fast_partials(g, v, d_vbar + t, sc->part32.p, &n_slabs, s);
-            IHTB_LAUNCH((k_sweep_epilogue<float>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part32.p, n_slabs,
-                        g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
-                        g->impute, out, (const float*)nullptr, fuse);
+    if (geno_is_dense(g)) {
+        // every mode computes the same exact FP64 product (dense.cu); a dense handle never pairs (d_l2 stays unused)
+        dense_xt_v(g, dV, m, dOut, s, &sc->part64, tf);
+    } else {
+        if (d_l2)
+            for (int64_t t = 0; t < m; ++t) IHTB_LAUNCH(k_l2norm, 1, 1024, 0, s, dV + t * g->n, g->n, d_vbar + t, d_l2 + t);
+        for (int64_t t = 0; t < m; ++t) {
+            const double* v = dV + t * g->n;
+            double* out = dOut + t * g->p;
+            if (mode == IHTB_SWEEP_PAIR && g->cs_j == 128 && t + 1 < m) {
+                // two right-hand sides per pass over the matrix (half2 tables); an odd last one takes the FAST path below
+                const int64_t n_slabs = sweep_fast_num_slabs(g);
+                if (sc->part32.n < (size_t)(2 * n_slabs * g->p)) sc->part32.alloc((size_t)(2 * n_slabs * g->p));
+                if (sc->scale.n < 2) sc->scale.alloc(2);
+                IHTB_LAUNCH(k_pair_scale, 1, 1024, 0, s, v, v + g->n, g->n, d_vbar + t, sc->scale.p);
+                sweep_pair_partials(g, v, v + g->n, d_vbar + t, sc->scale.p, sc->part32.p, s);
+                for (int h = 0; h < 2; ++h)
+                    IHTB_LAUNCH((k_sweep_epilogue<float>), (unsigned)ceil_div(g->p, 256), 256, 0, s,
+                                sc->part32.p + (size_t)h * n_slabs * g->p, n_slabs, g->p, g->mu.p, g->sinv.p, g->nmiss.p,
+                                g->miss_ptr.p, g->miss_idx.p, v + h * g->n, d_vbar + t + h, g->impute, out + h * g->p,
+                                sc->scale.p + h);
+                ++t;
+                continue;
+            }
+            if (mode == IHTB_SWEEP_EXACT && exact_uses_lut(g)) {
+                const int64_t n_slabs = g->stride / 128;
+                if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
+                sweep_exact_lut_partials(g, v, d_vbar + t, sc->part64.p, s);
+                IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
+                            g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
+                            g->impute, out, (const float*)nullptr, fuse);
+            } else if (mode == IHTB_SWEEP_EXACT) {
+                int64_t words = g->stride >> 2;
+                int64_t n_slabs = ceil_div(words, EX_THREADS);
+                if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
+                dim3 grid((unsigned)ceil_div(g->p, EX_COLS_PER_CTA), (unsigned)n_slabs);
+                IHTB_LAUNCH(k_sweep_exact, grid, EX_THREADS, 0, s, geno_view(g), v, d_vbar + t, sc->part64.p);
+                IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
+                            g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
+                            g->impute, out, (const float*)nullptr, fuse);
+            } else {
+                int64_t n_slabs = sweep_fast_num_slabs(g);
+                if (sc->part32.n < (size_t)(n_slabs * g->p)) sc->part32.alloc((size_t)(n_slabs * g->p));
+                sweep_fast_partials(g, v, d_vbar + t, sc->part32.p, &n_slabs, s);
+                IHTB_LAUNCH((k_sweep_epilogue<float>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part32.p, n_slabs,
+                            g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
+                            g->impute, out, (const float*)nullptr, fuse);
+            }
         }
     }
     if (sweep_ms) {
@@ -294,7 +299,7 @@ bool SweepPairer::sweep(int slot, const ihtb_geno* g, const double* d_v, const d
     const int other = slot ^ 1;
     IHTB_CUDA(cudaEventRecord(ready[slot], s));        // v / vbar of this fit are complete at this point of its stream
     std::unique_lock<std::mutex> lk(mu);
-    if (active >= 2 && g->cs_j == 128) {
+    if (active >= 2 && !geno_is_dense(g) && g->cs_j == 128) {
         req[slot] = Req{d_v, d_vbar, d_out, s};
         has[slot] = true;
         if (has[other]) {
@@ -402,7 +407,14 @@ extern "C" int32_t ihtb_sweep_bench(const ihtb_geno* g, int32_t sweep_mode, int3
         // (b) the dominant kernel alone
         if (ms_kernel) {
             *ms_kernel = 0.0;
-            if (sweep_mode == IHTB_SWEEP_PAIR) {
+            if (geno_is_dense(g)) {
+                IHTB_CUDA(cudaEventRecord(e0, s));
+                for (int i = 0; i < reps; ++i) dense_sweep_kernel_only(g, dV.p, &sc.part64, s);
+                IHTB_CUDA(cudaEventRecord(e1, s));
+                IHTB_CUDA(cudaEventSynchronize(e1));
+                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+                *ms_kernel = ms / reps;
+            } else if (sweep_mode == IHTB_SWEEP_PAIR) {
                 IHTB_CHECK(g->cs_j == 128, IHTB_EUNSUPPORTED, "the pair sweep needs a tiled layout");
                 IHTB_CUDA(cudaEventRecord(e0, s));
                 for (int i = 0; i < reps; ++i)
