@@ -39,8 +39,9 @@ void sweep_class_sums(const ihtb_geno* g, const double* d_v, double* d_w1, doubl
 using namespace ihtb;
 
 // worst-case absolute error of the FAST sweep's sum_i dosage_ij u_i, as a multiple of ||u||_1 :
-// 1 rounding of u to FP32 + 3 adds in the table (4 with the ternary tiles: five dosages per byte) + 3 adds per lane +
-// 5 butterfly adds = 13 roundings of at most 2^-24 relative on partial sums bounded by 2*||u||_1 (dosage <= 2)
+// 1 rounding of u to FP32 + 3 adds in the table (4 with the ternary tiles: five dosages per byte) + 3 adds per word +
+// 5 levels of the pairwise tree over a chunk's 32 words (butterfly or per-lane, sweep_lut.cu) = 13 roundings of at most
+// 2^-24 relative on partial sums bounded by 2*||u||_1 (dosage <= 2)
 // ->  13 * 2^-24 * 2 = 1.55e-6 ; we use 2^-18 = 3.8e-6 (2.5x margin).  The FP64 cross-slab sums add < 1e-13.
 static const double kFastBound = 1.0 / 262144.0;
 static const double kExactBound = 1e-13;

@@ -46,6 +46,14 @@ __device__ __forceinline__ uint4 lds_u128(uint32_t addr) {
     asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
     return v;
 }
+// byte permute with the selector as an immediate: unlike __byte_perm, a selector nibble with bit 3 set replicates the
+// sign bit of the selected byte (0x00 for a byte below 0x80)
+template <uint32_t SEL>
+__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b) {
+    uint32_t d;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "n"(SEL));
+    return d;
+}
 __device__ __forceinline__ void sts_u32(uint32_t addr, uint32_t v) {
     asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
 }
