@@ -157,16 +157,34 @@ int32_t ihtb_geno_destroy(ihtb_geno* g);
  *   sum), sigma_j = sqrt(mu_j (1 - mu_j/2)), missing -> mu_j, x = (g - mu_j) * (1/sigma_j) (1/sigma_j = 1 if sigma_j = 0):
  *   integer dosages give the bits of ihtb_geno_decode of the same genotypes in a PLINK handle.
  * On a DENSE handle ihtb_geno_stats returns the mu / sigma_inv / missing counts applied (0 / 1 / 0 with standardize = 0),
- * ihtb_geno_decode the stored values, ihtb_geno_sweep_stream_bytes n*p*sizeof(T) with ternary = 0; ihtb_geno_packed,
+ * ihtb_geno_decode the stored values, ihtb_geno_sweep_stream_bytes n*p*sizeof(T) with ternary = 0 (2*n*p for
+ * IHTB_DENSE_FIX16 below); ihtb_geno_packed,
  * counts, maf, ternary_tiles, gather_bench and set_offset return IHTB_EUNSUPPORTED and load_columns IHTB_EINVAL.
  * Not supported on a DENSE handle (IHTB_EUNSUPPORTED): multivariate fits, SNP-sharded fits, multi-device handles. */
-enum { IHTB_DENSE_F64 = 0, IHTB_DENSE_F32 = 1 };
+enum { IHTB_DENSE_F64 = 0, IHTB_DENSE_F32 = 1, IHTB_DENSE_FIX16 = 2 };
+/* dtype IHTB_DENSE_F64 or IHTB_DENSE_F32 (IHTB_DENSE_FIX16 needs a denominator: ihtb_geno_create_dosage16) */
 int32_t ihtb_geno_create_dense(const void* x, int32_t dtype, int64_t n, int64_t p, int64_t ld, int32_t standardize,
                                ihtb_geno** out);
 /* piecewise form: create_dense_empty, load_dense_columns for columns [j_first, j_first+ncols) (any order, each column
- * once; x + c*ld is column j_first + c), then ihtb_geno_finalize */
+ * once; x + c*ld is column j_first + c, elements of the handle's storage type), then ihtb_geno_finalize */
 int32_t ihtb_geno_create_dense_empty(int64_t n, int64_t p, int32_t dtype, int32_t standardize, ihtb_geno** out);
 int32_t ihtb_geno_load_dense_columns(ihtb_geno* g, const void* x, int64_t ld, int64_t j_first, int64_t ncols);
+/* Dosages on a fixed-point grid (IHTB_DENSE_FIX16): uint16_t codes, code c stands for the value c / denominator,
+ * 1 <= denominator <= 65534 (PLINK 2 dosages: 16384; VCF DS printed with d decimals: 10^d; BGEN 8-bit: 255).  Code
+ * IHTB_DOSAGE16_MISSING is a missing entry: allowed only with standardize = 1 (where it plays the role of NaN), otherwise
+ * IHTB_EDOMAIN at finalize.  Storage is 2 bytes per entry, and the handle computes exactly what a Float64 handle of the
+ * decoded values computes: every kernel that reads an entry uses g = c / D (IEEE FP64 division) and, standardized,
+ * x = (g - mu_j) * sigma_inv_j with the operations above; mu_j, sigma_inv_j and the missing counts come out bit for bit
+ * those of the Float64 handle.  So ihtb_geno_decode, ihtb_geno_stats, the support matvec, the re-scoring and with them
+ * the fitted support, iterations, beta, c and logl equal those of ihtb_geno_create_dense(c / D as FP64, standardize).
+ * The X'v sweep reads the codes (ihtb_geno_sweep_stream_bytes: 2 n p) and centres / scales in its epilogue; its values
+ * differ from the Float64 handle's in the last bits, within the documented selection bound.  Columns load through
+ * ihtb_geno_load_dense_columns (uint16_t elements) followed by ihtb_geno_finalize. */
+enum { IHTB_DOSAGE16_MISSING = 65535 };
+int32_t ihtb_geno_create_dosage16(const uint16_t* codes, int64_t n, int64_t p, int64_t ld, int32_t denominator,
+                                  int32_t standardize, ihtb_geno** out);
+int32_t ihtb_geno_create_dosage16_empty(int64_t n, int64_t p, int32_t denominator, int32_t standardize,
+                                        ihtb_geno** out);
 
 /* ---- univariate fit (fit_iht / fit_iht! / init_iht_indices!, src/fit.jl:60-207, src/utilities.jl:366-438) ---- */
 /* y[n]; z is n x q column-major with the intercept in column 0; zkeep[q] (0/1) or NULL for all kept. */

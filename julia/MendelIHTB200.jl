@@ -99,23 +99,56 @@ Base.size(x::B200MultiSnpLinAlg) = (x.n, x.p)
 # ---- dense design matrix (include/ihtb200.h ihtb_geno_create_dense) ----------------------------------------------
 """Device-resident dense predictors: `fit_iht(y, x::AbstractMatrix{T}, z)` (src/fit.jl:62) for T = Float64 / Float32,
 e.g. the dosages `convert_gt` / `convert_bgen_gt` produce (src/wrapper.jl:406-485).  `standardize = true` runs
-`standardize_genotypes!` on the device (NaN = missing).  Stored as T, computed on in Float64; univariate fits only."""
+`standardize_genotypes!` on the device (NaN = missing).  Stored as T, computed on in Float64; univariate fits only.
+
+`dosage_denominator = D` (Float64 input, 1 <= D <= 65534): dosages on the grid 1/D (PLINK 2: 16384, VCF DS with d
+decimals: 10^d, BGEN 8-bit: 255) are stored losslessly as 16-bit codes c = round(x D), 2 bytes per entry; every entry
+must satisfy 0 <= c <= 65534 and c / D == x (ArgumentError otherwise), NaN is missing with `standardize = true`.  Results
+equal those of the Float64 storage of the same values (include/ihtb200.h ihtb_geno_create_dosage16)."""
 mutable struct B200DenseLinAlg{T<:Union{Float32,Float64}} <: AbstractMatrix{T}
     handle::Ptr{Cvoid}
     n::Int
     p::Int
-    function B200DenseLinAlg(x::Matrix{T}; standardize::Bool=false) where {T<:Union{Float32,Float64}}
+    function B200DenseLinAlg(x::Matrix{T}; standardize::Bool=false,
+                             dosage_denominator::Union{Nothing,Integer}=nothing) where {T<:Union{Float32,Float64}}
         n, p = size(x)
         h = Ref{Ptr{Cvoid}}(C_NULL)
-        check(ccall((:ihtb_geno_create_dense, LIB), Int32,
-                    (Ptr{Cvoid}, Int32, Int64, Int64, Int64, Int32, Ref{Ptr{Cvoid}}),
-                    x, T === Float32 ? 1 : 0, n, p, n, standardize, h))
+        if dosage_denominator === nothing
+            check(ccall((:ihtb_geno_create_dense, LIB), Int32,
+                        (Ptr{Cvoid}, Int32, Int64, Int64, Int64, Int32, Ref{Ptr{Cvoid}}),
+                        x, T === Float32 ? 1 : 0, n, p, n, standardize, h))
+        else
+            codes = encode_dosages(x, dosage_denominator, standardize)
+            check(ccall((:ihtb_geno_create_dosage16, LIB), Int32,
+                        (Ptr{UInt16}, Int64, Int64, Int64, Int32, Int32, Ref{Ptr{Cvoid}}),
+                        codes, n, p, n, dosage_denominator, standardize, h))
+        end
         g = new{T}(h[], n, p)
         finalizer(g -> ccall((:ihtb_geno_destroy, LIB), Int32, (Ptr{Cvoid},), g.handle), g)
         return g
     end
 end
 Base.size(x::B200DenseLinAlg) = (x.n, x.p)
+
+# codes c = round(x D) of dosages on the grid 1/D; the first entry (column-major) that is not c / D names the error
+function encode_dosages(x::Matrix{T}, D::Integer, standardize::Bool) where {T}
+    T === Float64 || throw(ArgumentError("dosage codes need Float64 input"))
+    1 <= D <= 65534 || throw(ArgumentError("dosage_denominator must be in [1, 65534], got $D"))
+    codes = Matrix{UInt16}(undef, size(x))
+    @inbounds for j in axes(x, 2), i in axes(x, 1)
+        v = x[i, j]
+        if isnan(v)
+            standardize || throw(DomainError(v, "x[$i, $j] is NaN: missing dosages need standardize = true"))
+            codes[i, j] = 0xffff
+            continue
+        end
+        c = round(v * D)
+        (0 <= c <= 65534 && c / D == v) ||
+            throw(ArgumentError("x[$i, $j] = $v is not a dosage c / $D with an integer 0 <= c <= 65534"))
+        codes[i, j] = UInt16(c)
+    end
+    codes
+end
 function Base.getindex(x::B200DenseLinAlg{T}, i::Int, j::Int) where {T}     # the stored value
     out = Ref{Float64}(0.0)
     check(ccall((:ihtb_geno_decode, LIB), Int32, (Ptr{Cvoid}, Int64, Int64, Int64, Int64, Ref{Float64}),

@@ -17,7 +17,8 @@ LIB_PATH = os.path.join(HERE, "libihtb200.so")
 IHTB_OK, IHTB_EINVAL, IHTB_EDIM, IHTB_EDOMAIN, IHTB_ENUMERIC, IHTB_ECUDA, IHTB_ENOMEM, IHTB_EUNSUPPORTED = (
     0, -1, -2, -3, -4, -5, -6, -7)
 SWEEP_FAST, SWEEP_EXACT, SWEEP_PAIR = 0, 1, 2
-DENSE_F64, DENSE_F32 = 0, 1
+DENSE_F64, DENSE_F32, DENSE_FIX16 = 0, 1, 2
+DOSAGE16_MISSING = 65535
 
 
 class IHTBError(RuntimeError):
@@ -94,6 +95,8 @@ SIGNATURES = {
     "ihtb_geno_create_dense": [_p, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _pp],
     "ihtb_geno_create_dense_empty": [C.c_int64, C.c_int64, C.c_int32, C.c_int32, _pp],
     "ihtb_geno_load_dense_columns": [_p, _p, C.c_int64, C.c_int64, C.c_int64],
+    "ihtb_geno_create_dosage16": [_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, _pp],
+    "ihtb_geno_create_dosage16_empty": [C.c_int64, C.c_int64, C.c_int32, C.c_int32, _pp],
     "ihtb_fit_create": [_p, _f64, _f64, C.c_int64, _u8, C.POINTER(Cfg), _pp],
     "ihtb_fit_create_sharded": [_p, _p, C.c_int64, _f64, _f64, C.c_int64, _u8, C.POINTER(Cfg), _pp],
     "ihtb_fit_set_weights": [_p, _f64],

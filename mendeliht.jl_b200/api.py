@@ -191,18 +191,20 @@ class B200SnpLinAlg:
 
 
 class B200DenseLinAlg:
-    """Device-resident dense n x p design matrix (float64 or float32 entries, computed on in FP64): imputed dosages from
+    """Device-resident dense n x p design matrix (float64 or float32 entries, or 16-bit fixed-point dosage codes from
+    `from_dosages`; computed on in FP64): imputed dosages from
     VCF / BGEN or any real predictors.  Works wherever a single-GPU `B200SnpLinAlg` does in `fit_iht`, `cv_iht`, `cv_run`
     and `IHTVariable` (univariate traits)."""
 
     # host memory of the column-block upload of a C-ordered array (one block at a time)
     _BLOCK_BYTES = 64 << 20
 
-    def __init__(self, handle, n, p, dtype, standardize):
+    def __init__(self, handle, n, p, dtype, standardize, denominator=None):
         self._h = handle
         self.n, self.p = int(n), int(p)
         self.dtype = np.dtype(dtype)
         self.standardize = bool(standardize)
+        self.denominator = denominator
 
     @classmethod
     def from_array(cls, x: np.ndarray, standardize: bool = False) -> "B200DenseLinAlg":
@@ -240,6 +242,68 @@ class B200DenseLinAlg:
         check(lib.ihtb_geno_finalize(h))
         return obj
 
+    @staticmethod
+    def encode_dosages(x: np.ndarray, denominator: int, standardize: bool = False) -> np.ndarray:
+        """The uint16 codes c = rint(x * D) of a float64 block, checked to be exact: every non-NaN entry must satisfy
+        0 <= c <= 65534 and c / D == x; NaN becomes the missing code 65535 when standardizing.  Raises ValueError
+        naming the first offending (i, j) (column-major order) and its value, IHTBError(IHTB_EDOMAIN) for NaN without
+        standardization."""
+        miss = np.isnan(x)
+        if miss.any() and not standardize:
+            i, j = _first_true(miss)
+            raise _lib.IHTBError(_lib.IHTB_EDOMAIN, f"x[{i}, {j}] is NaN: missing dosages need standardize=True")
+        xs = np.where(miss, 0.0, x)
+        with np.errstate(invalid="ignore", over="ignore"):
+            c = np.rint(xs * denominator)
+            bad = ~((c >= 0) & (c <= 65534))
+            c = np.where(bad, 0.0, c)
+            bad |= c / denominator != xs
+        if bad.any():
+            i, j = _first_true(bad)
+            raise ValueError(f"x[{i}, {j}] = {float(x[i, j])!r} is not a dosage c / {denominator} with an integer "
+                             f"0 <= c <= 65534")
+        codes = c.astype(np.uint16)
+        codes[miss] = _lib.DOSAGE16_MISSING
+        return codes
+
+    @classmethod
+    def from_dosages(cls, x: np.ndarray, denominator: int, standardize: bool = False) -> "B200DenseLinAlg":
+        """Lossless 16-bit fixed-point storage of dosages that lie on the grid 1 / denominator (PLINK 2: 16384, VCF DS
+        printed with d decimals: 10**d, BGEN 8-bit: 255; 1 <= denominator <= 65534).  x: float64 ndarray [n, p] in any
+        layout, encoded on the host in column blocks as code c = rint(x * D) (every entry is checked: c / D == x
+        exactly).  NaN is missing with standardize=True and an IHTBError(IHTB_EDOMAIN) otherwise, as in `from_array`.
+        The device holds 2 bytes per entry, and every result (decode, stats, fits, cross-validation) is that of
+        `from_array(x, standardize)` bit for bit; the X'v sweep reads the codes and differs only in the last bits,
+        within its selection bound.  `dtype` is uint16."""
+        if not isinstance(x, np.ndarray):
+            raise TypeError("x must be a numpy ndarray")
+        if x.ndim != 2:
+            raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"x must be a matrix (ndim 2), got ndim {x.ndim}")
+        if x.dtype != np.float64:
+            raise TypeError(f"x must be float64, got {x.dtype}")
+        if isinstance(denominator, (bool, np.bool_)) or not isinstance(denominator, (int, np.integer)):
+            raise TypeError(f"denominator must be an integer, got {type(denominator).__name__}")
+        denominator = int(denominator)
+        if not 1 <= denominator <= 65534:
+            raise ValueError(f"denominator must be in [1, 65534], got {denominator}")
+        n, p = x.shape
+        if n == 0 or p == 0:
+            raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"x must have n > 0 and p > 0, got {x.shape}")
+        cols = max(1, cls._BLOCK_BYTES // (n * 8))
+        # the first block is checked before the device is touched (all of a matrix up to 64 MB); a bad entry in a later
+        # block raises before that block is uploaded, and the handle is released with `obj`
+        first = cls.encode_dosages(x[:, :cols], denominator, standardize)
+        lib = load()
+        h = C.c_void_p()
+        check(lib.ihtb_geno_create_dosage16_empty(n, p, denominator, int(bool(standardize)), C.byref(h)))
+        obj = cls(h, n, p, np.uint16, standardize, denominator)
+        for j in range(0, p, cols):
+            blk = first if j == 0 else cls.encode_dosages(x[:, j:j + cols], denominator, standardize)
+            blk = np.asfortranarray(blk)
+            check(lib.ihtb_geno_load_dense_columns(h, C.c_void_p(blk.ctypes.data), n, j, blk.shape[1]))
+        check(lib.ihtb_geno_finalize(h))
+        return obj
+
     @property
     def shape(self):
         return (self.n, self.p)
@@ -264,7 +328,7 @@ class B200DenseLinAlg:
         return B200SnpLinAlg.x_support(self, idx, coef)
 
     def sweep_stream_bytes(self):
-        """(bytes one X'v sweep reads from HBM = n p sizeof(T), False)"""
+        """(bytes one X'v sweep reads from HBM = n p sizeof(T), 2 n p for dosage codes, False)"""
         return B200SnpLinAlg.sweep_stream_bytes(self)
 
     def close(self):
@@ -277,6 +341,12 @@ class B200DenseLinAlg:
             self.close()
         except Exception:
             pass
+
+
+def _first_true(mask: np.ndarray):
+    """(i, j) of the first True entry of a 2-D mask in column-major order"""
+    j = int(np.flatnonzero(mask.any(axis=0))[0])
+    return int(np.flatnonzero(mask[:, j])[0]), j
 
 
 class B200MultiSnpLinAlg:

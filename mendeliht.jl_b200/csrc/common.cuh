@@ -128,7 +128,7 @@ static inline void ensure_dynamic_smem(K kernel, int bytes) {
 // ---- genotype handle -----------------------------------------------------------------------
 struct TopkFuse;
 // dense.cu (DENSE handles).  The dense X'v is the plain product sum_i x_ij v_i: no centring, the mean of v is not read.
-ihtb_geno* dense_new_handle(int64_t n, int64_t p, int dtype, int standardize);
+ihtb_geno* dense_new_handle(int64_t n, int64_t p, int dtype, int standardize, int32_t den = 0);
 void dense_upload(ihtb_geno* g, const void* x, int64_t ld_host, int64_t j_dst, int64_t ncols);
 void dense_finalize(ihtb_geno* g);       // statistics / standardization, error-bound scale; IHTB_EDOMAIN on bad entries
 int64_t dense_stream_bytes(const ihtb_geno* g);
@@ -191,17 +191,19 @@ struct ihtb_geno {
     // sqrt(sum_i g_ij^2) * ||u||_2 (Cauchy-Schwarz), which is far tighter than 2 ||u||_1 for the PAIR sweep
     ihtb::DBuf<double> sgn;
     ihtb::DBuf<int32_t> nmiss;
-    // CSR of missing samples per column (sparse imputation correction of the sweep)
+    // CSR of missing samples per column (sparse imputation correction of the sweep; PLINK and standardized FIX16 handles)
     ihtb::DBuf<int64_t> miss_ptr;   // [p+1]
     ihtb::DBuf<int32_t> miss_idx;   // sample indices
     int64_t total_missing = 0;
     bool ready = false;             // columns loaded and statistics computed (false between create_empty and finalize)
     // ---- DENSE handles (dense.cu) ----
-    int dtype = 0;                  // IHTB_DENSE_F64 | IHTB_DENSE_F32
-    int standardize = 0;            // 1: standardize_genotypes! applied at finalize (NaN = missing)
+    int dtype = 0;                  // IHTB_DENSE_F64 | IHTB_DENSE_F32 | IHTB_DENSE_FIX16
+    int standardize = 0;            // 1: standardize_genotypes! applied at finalize (NaN / the missing code = missing)
+    int32_t den = 0;                // FIX16: code c stands for c / den (1..65534); 0 for float storage
     int64_t ld = 0;                 // device leading dimension in elements: n rounded up to a whole number of sweep slabs
     ihtb::DBuf<uint8_t> dense;      // p * ld elements, zero padded below row n
-    ihtb::DBuf<double> dscale;      // per-column error-bound scale max_i |x_ij| of the stored (standardized) matrix
+    // per-column error-bound scale: max_i |x_ij| of the stored (standardized) matrix; FIX16 dense_finalize
+    ihtb::DBuf<double> dscale;
     double dcoef = 0.0;             // error-bound coefficient of the dense sweep + re-scoring (dense_bound_coef)
 };
 static inline bool geno_is_dense(const ihtb_geno* g) { return g->kind == GENO_DENSE; }
