@@ -185,6 +185,27 @@ int32_t ihtb_geno_create_dosage16(const uint16_t* codes, int64_t n, int64_t p, i
                                   int32_t standardize, ihtb_geno** out);
 int32_t ihtb_geno_create_dosage16_empty(int64_t n, int64_t p, int32_t denominator, int32_t standardize,
                                         ihtb_geno** out);
+/* BGEN 1.2 dosages (layout 2): columns [j_first, j_first+ncols) of an unfinalized IHTB_DENSE_FIX16 or IHTB_DENSE_F64
+ * handle from the INFLATED probability blocks of ncols variants (decompression stays with the caller).  Block c is
+ * blocks[offsets[c] .. offsets[c+1]) (offsets has ncols + 1 entries, non-decreasing) and becomes column j_first + c.
+ * A block is uint32 N, uint16 K, uint8 Pmin, Pmax, N ploidy bytes (bit 7 = missing), uint8 phased, uint8 B, then 2 N
+ * B-bit values packed least-significant bit first.  With D = 2^B - 1 the dosage of the second allele is code / D,
+ * code = b + 2 (D - a - b) unphased (a = P(11), b = P(12)) or 2 D - h1 - h2 phased; allele = 1 counts the first allele
+ * (2 D - code).  FIX16 handles store the code and need D == the handle's denominator (so B <= 15); F64 handles store
+ * code / D (IEEE FP64 division, any B).  A missing sample is stored as IHTB_DOSAGE16_MISSING / NaN, so it needs
+ * standardize = 1 at ihtb_geno_finalize, as for the other loaders.  The blocks are staged through two pinned buffers
+ * and decoded on the device (one CTA per block).  Errors name the LOWEST failing block and the reason:
+ *   IHTB_EDIM         block N != n
+ *   IHTB_EUNSUPPORTED K != 2, or ploidy != 2 on a non-missing sample
+ *   IHTB_EINVAL       B = 0, B > 32, 2^B - 1 != the FIX16 denominator, phased flag not 0 / 1, a block shorter than its
+ *                     header + ceil(2 N B / 8) bytes; an F32 handle, allele not 1 / 2, decreasing offsets
+ *   IHTB_EDOMAIN      unphased a + b > D
+ * After an error the contents of the columns of this call are unspecified (load them again or destroy the handle). */
+int32_t ihtb_geno_load_bgen_columns(ihtb_geno* g, const uint8_t* blocks, const int64_t* offsets, int64_t j_first,
+                                    int64_t ncols, int32_t allele);
+/* Host staging batch of ihtb_geno_load_bgen_columns in bytes (whole blocks, at least one per batch; default 64 MiB,
+ * restored by bytes <= 0).  Process-wide; a tuning and test knob. */
+int32_t ihtb_bgen_set_batch_bytes(int64_t bytes);
 
 /* ---- univariate fit (fit_iht / fit_iht! / init_iht_indices!, src/fit.jl:60-207, src/utilities.jl:366-438) ---- */
 /* y[n]; z is n x q column-major with the intercept in column 0; zkeep[q] (0/1) or NULL for all kept. */

@@ -97,6 +97,8 @@ SIGNATURES = {
     "ihtb_geno_load_dense_columns": [_p, _p, C.c_int64, C.c_int64, C.c_int64],
     "ihtb_geno_create_dosage16": [_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, _pp],
     "ihtb_geno_create_dosage16_empty": [C.c_int64, C.c_int64, C.c_int32, C.c_int32, _pp],
+    "ihtb_geno_load_bgen_columns": [_p, _u8, _i64, C.c_int64, C.c_int64, C.c_int32],
+    "ihtb_bgen_set_batch_bytes": [C.c_int64],
     "ihtb_fit_create": [_p, _f64, _f64, C.c_int64, _u8, C.POINTER(Cfg), _pp],
     "ihtb_fit_create_sharded": [_p, _p, C.c_int64, _f64, _f64, C.c_int64, _u8, C.POINTER(Cfg), _pp],
     "ihtb_fit_set_weights": [_p, _f64],

@@ -4,15 +4,18 @@ Same names, argument meaning and error behaviour as the reference (all paths und
   `B200SnpLinAlg`  <- `SnpLinAlg{Float64}(s; model=ADDITIVE_MODEL, center, scale, impute)`  src/wrapper.jl:68-69
   `B200DenseLinAlg` <- a dense `x::AbstractMatrix{T}`, T = Float64 / Float32  src/fit.jl:62 (standardize_genotypes!,
                        src/wrapper.jl:406-423, on the device when asked)
+                       `from_bgen` <- the dense dosages `parse_genotypes` reads from .bgen  src/wrapper.jl:451-485
   `fit_iht`        <- src/fit.jl:60-118        `IHTResult` <- src/data_structures.jl:245-258
   `cv_iht`         <- src/cross_validation.jl:60-131
-  `iht`            <- src/wrapper.jl:52-120    `cross_validate` <- src/wrapper.jl:301-349
+  `iht`            <- src/wrapper.jl:52-120    `cross_validate` <- src/wrapper.jl:301-349  (PLINK or .bgen input)
 Julia is not available in this image, so this Python layer plays the role of julia/MendelIHTB200.jl (which binds
 the very same C entry points with ccall); every numerical step happens inside the CUDA library.
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
+from concurrent.futures import ThreadPoolExecutor
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -302,6 +305,103 @@ class B200DenseLinAlg:
             blk = np.asfortranarray(blk)
             check(lib.ihtb_geno_load_dense_columns(h, C.c_void_p(blk.ctypes.data), n, j, blk.shape[1]))
         check(lib.ihtb_geno_finalize(h))
+        return obj
+
+    @classmethod
+    def from_bgen(cls, paths, standardize: bool = False, allele: int = 2, storage: str = "auto") -> "B200DenseLinAlg":
+        """Dosages of BGEN 1.2 files (layout 2, uncompressed or zlib; biallelic diploid variants).  `paths`: one file or
+        a list (e.g. one per chromosome) over the same samples -- N must match, and so must the sample IDs where files
+        carry them -- whose variants become the columns in the order given.  A probability stored as a B-bit integer
+        makes the dosage of `allele` (2, the default: copies of the second allele, what a PLINK handle counts; or 1)
+        exactly code / (2^B - 1); the host inflates the blocks (thread pool, ~64 MB batches) and the device decodes them
+        (ihtb_geno_load_bgen_columns).  storage="auto": 16-bit codes with denominator 2^B - 1 (as `from_dosages`) when
+        the first variant has B <= 15, Float64 otherwise; "fix16" / "f64" force one (a FIX16 handle needs the same B in
+        every variant).  Missing samples need standardize=True, as NaN does for `from_array`.  The handle equals
+        `from_dosages(codes / D, D, standardize)` (FIX16) or `from_array(codes / D, standardize)` bit for bit
+        (bgen.dosage_codes is the host twin), and carries `.variants` (bgen.BgenVariant per column) and `.samples`
+        (sample IDs, or None when no file stores them)."""
+        from . import bgen as _bgen
+        if isinstance(paths, (str, bytes, os.PathLike)):
+            paths = [paths]
+        paths = [os.fspath(q) for q in paths]
+        if not paths:
+            raise ValueError("from_bgen needs at least one file")
+        if isinstance(allele, (bool, np.bool_)) or allele not in (1, 2):
+            raise ValueError(f"allele must be 1 or 2, got {allele!r}")
+        if storage not in ("auto", "fix16", "f64"):
+            raise ValueError(f"storage must be 'auto', 'fix16' or 'f64', got {storage!r}")
+        files = []
+        try:
+            for q in paths:
+                files.append(_bgen.BgenFile(q))
+            n = files[0].n
+            samples, samples_from = None, None
+            for f in files:
+                if f.n != n:
+                    raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"{f.path} holds {f.n} samples, {files[0].path} {n}")
+                if f.samples is not None:
+                    if samples is None:
+                        samples, samples_from = f.samples, f.path
+                    elif f.samples != samples:
+                        raise ValueError(f"{f.path}: sample identifiers differ from those of {samples_from}")
+            p = sum(f.m for f in files)
+            if n == 0 or p == 0:
+                raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"BGEN input must have n > 0 samples and p > 0 variants, "
+                                                             f"got n = {n}, p = {p}")
+            variants = [v for f in files for v in f.variants]
+            jobs, j = [], 0
+            for f in files:
+                for c0, c1 in f.batches(_bgen.INFLATE_BATCH_BYTES):
+                    jobs.append((f, c0, c1, j + c0))
+                j += f.m
+            return cls._load_bgen(jobs, n, p, variants, samples, standardize, allele, storage)
+        finally:
+            for f in files:
+                f.close()
+
+    @classmethod
+    def _load_bgen(cls, jobs, n, p, variants, samples, standardize, allele, storage):
+        from . import bgen as _bgen
+        lib = load()
+        obj = None
+        with ThreadPoolExecutor(max_workers=max(1, min(32, os.cpu_count() or 1))) as pool, \
+                ThreadPoolExecutor(max_workers=1) as ahead:
+            def inflate(job):
+                f, c0, c1, _ = job
+                return f.inflate(c0, c1, pool)
+            nxt = ahead.submit(inflate, jobs[0])
+            for t, job in enumerate(jobs):
+                buf, offs = nxt.result()
+                if t + 1 < len(jobs):
+                    nxt = ahead.submit(inflate, jobs[t + 1])       # inflate the next batch while this one loads
+                f, c0, c1, jcol = job
+                bits = _bgen.block_bits(buf, offs, n)
+                if obj is None:
+                    b0 = int(bits[0])
+                    if storage == "fix16" and not 1 <= b0 <= 15:
+                        raise ValueError(f"{f.path}: variant {variants[0].name()} stores B = {b0} bits per probability; "
+                                         f"16-bit codes need B <= 15 (use storage='f64')")
+                    h = C.c_void_p()
+                    if storage == "fix16" or (storage == "auto" and 1 <= b0 <= 15):
+                        den = (1 << b0) - 1
+                        check(lib.ihtb_geno_create_dosage16_empty(n, p, den, int(bool(standardize)), C.byref(h)))
+                        obj = cls(h, n, p, np.uint16, standardize, den)
+                    else:
+                        check(lib.ihtb_geno_create_dense_empty(n, p, _lib.DENSE_F64, int(bool(standardize)), C.byref(h)))
+                        obj = cls(h, n, p, np.float64, standardize)
+                    obj.variants, obj.samples = variants, samples
+                if obj.denominator is not None:
+                    other = np.flatnonzero(bits != b0)
+                    if other.size:
+                        c = c0 + int(other[0])
+                        raise ValueError(f"{f.path}: variant {f.variants[c].name()} stores B = {int(bits[other[0]])} "
+                                         f"bits per probability, the first variant B = {b0}: 16-bit codes need one B "
+                                         f"for all variants (use storage='f64')")
+                status = lib.ihtb_geno_load_bgen_columns(obj._h, _lib.ptr(buf, C.c_uint8), _lib.ptr(offs, C.c_int64),
+                                                         jcol, c1 - c0, int(allele))
+                if status != _lib.IHTB_OK:
+                    raise _lib._EXC.get(status, _lib.IHTBError)(status, f"{f.path}: {_lib.last_error()}")
+        check(lib.ihtb_geno_finalize(obj._h))
         return obj
 
     @property
@@ -956,12 +1056,43 @@ def _load_plink(filename: str, phenotypes, d: str):
     return x, y
 
 
+def _bgen_input(filename: str):
+    """The BGEN file that `filename` names (it ends in .bgen, or it is a prefix with prefix.bgen and no prefix.bed),
+    else None: PLINK input keeps precedence."""
+    fn = os.fspath(filename)
+    if fn.endswith(".bgen"):
+        return fn
+    if not os.path.exists(fn + ".bed") and os.path.exists(fn + ".bgen"):
+        return fn + ".bgen"
+    return None
+
+
+def _load_input(filename: str, phenotypes, d: str):
+    """(x, y) of PLINK or BGEN input.  BGEN dosages are standardized like the reference's dense dosages
+    (src/wrapper.jl:406-423); a BGEN file has no .fam, so phenotypes is an array or a comma-separated file."""
+    path = _bgen_input(filename)
+    if path is None:
+        return _load_plink(filename, phenotypes, d)
+    if isinstance(phenotypes, (bool, int, np.integer)):
+        raise ValueError(f"{path}: BGEN input has no .fam file to take phenotype column {phenotypes} from; pass "
+                         f"phenotypes as an array or a comma-separated file")
+    if isinstance(phenotypes, (list, tuple, np.ndarray)):
+        y = np.asarray(phenotypes, dtype=np.float64)
+    else:
+        y = np.loadtxt(phenotypes, delimiter=",", dtype=np.float64)
+        if y.ndim == 2:
+            y = np.ascontiguousarray(y.T) if y.shape[1] > 1 else y[:, 0]
+    return B200DenseLinAlg.from_bgen(path, standardize=True), y
+
+
 def iht(filename: str, k: int, d: str = NORMAL, phenotypes=6, covariates: str = "", summaryfile: str = None,
         betafile: str = None, exclude_std_idx=(), **kwargs) -> IHTResult:
     """`iht(filename, k, d; phenotypes, covariates, ...)` (src/wrapper.jl:52-120) for binary PLINK input: reads
     `filename`.bed/.fam, builds the device genotype operator with center/scale/impute, standardises covariates and
-    runs `fit_iht` with the canonical link (LogLink for NegativeBinomial).  Optional text outputs like the reference."""
-    x, y = _load_plink(filename, phenotypes, d)
+    runs `fit_iht` with the canonical link (LogLink for NegativeBinomial).  Optional text outputs like the reference.
+    BGEN input: `filename` ending in .bgen (or a prefix with prefix.bgen and no prefix.bed) is read with
+    `B200DenseLinAlg.from_bgen(standardize=True)`; `phenotypes` is then an array or a comma-separated file."""
+    x, y = _load_input(filename, phenotypes, d)
     z = np.ones(x.n) if covariates == "" else parse_covariates(covariates, exclude_std_idx)
     if is_multivariate(y):          # src/wrapper.jl:80,84-85: z is transposed to q x n, no distribution / link
         z = np.ones((1, x.n)) if covariates == "" else np.ascontiguousarray(np.asarray(z).reshape(x.n, -1).T)
@@ -983,8 +1114,8 @@ def iht(filename: str, k: int, d: str = NORMAL, phenotypes=6, covariates: str = 
 
 def cross_validate(filename: str, d: str = NORMAL, path=range(1, 21), q: int = 5, phenotypes=6, covariates: str = "",
                    cv_summaryfile: str = None, exclude_std_idx=(), folds=None, **kwargs) -> np.ndarray:
-    """`cross_validate(filename, d; path, q, ...)` (src/wrapper.jl:301-349) for binary PLINK input."""
-    x, y = _load_plink(filename, phenotypes, d)
+    """`cross_validate(filename, d; path, q, ...)` (src/wrapper.jl:301-349) for binary PLINK or BGEN input (as `iht`)."""
+    x, y = _load_input(filename, phenotypes, d)
     z = np.ones(x.n) if covariates == "" else parse_covariates(covariates, exclude_std_idx)
     if is_multivariate(y):
         z = np.ones((1, x.n)) if covariates == "" else np.ascontiguousarray(np.asarray(z).reshape(x.n, -1).T)

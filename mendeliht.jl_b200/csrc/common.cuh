@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <memory>
 #include <string>
 #include <vector>
 #include <stdexcept>
@@ -205,6 +206,9 @@ struct ihtb_geno {
     // per-column error-bound scale: max_i |x_ij| of the stored (standardized) matrix; FIX16 dense_finalize
     ihtb::DBuf<double> dscale;
     double dcoef = 0.0;             // error-bound coefficient of the dense sweep + re-scoring (dense_bound_coef)
+    // staging buffers and streams of ihtb_geno_load_bgen_columns (bgen.cu), kept between its calls so that pinned memory
+    // is allocated once per load rather than once per batch; released at finalize
+    std::shared_ptr<void> bgen_stage;
 };
 static inline bool geno_is_dense(const ihtb_geno* g) { return g->kind == GENO_DENSE; }
 

@@ -731,6 +731,7 @@ static void fix16_missing_rows(ihtb_geno* g, int64_t* max_nmiss) {
 }
 
 void dense_finalize(ihtb_geno* g) {
+    g->bgen_stage.reset();
     g->mu.alloc(g->p); g->sinv.alloc(g->p); g->nmiss.alloc(g->p); g->dscale.alloc(g->p);
     DBuf<unsigned long long> bad(1);
     bad.zero(0);
