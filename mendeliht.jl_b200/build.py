@@ -10,7 +10,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libihtb200.so")
-SOURCES = ["geno.cu", "dense.cu", "bgen.cu", "support.cu", "sweep.cu", "sweep_lut.cu", "sweep_tmem.cu", "sweep_lut64.cu", "glm.cu", "topk.cu", "fit.cu", "comm.cu", "mvfit.cu", "p2p.cu", "debias.cu", "groups.cu", "multi.cu"]
+SOURCES = ["geno.cu", "dense.cu", "bgen.cu", "support.cu", "sweep.cu", "sweep_lut.cu", "sweep_lut64.cu", "glm.cu", "topk.cu", "fit.cu", "comm.cu", "mvfit.cu", "p2p.cu", "debias.cu", "groups.cu", "multi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

@@ -166,15 +166,13 @@ struct ihtb_geno {
     int64_t j0 = 0;           // global index of local column 0 (SNP-sharded fits)
     int64_t nbytes = 0;       // ceil(n/4)
     int64_t stride = 0;       // padded bytes per column: multiple of 128 (= 512-sample slabs), zero padded
-    // Byte b of column j lives at bed + j*cs_j + (b>>7)*cs_s + (b&127):
-    //   column-major: cs_j = stride, cs_s = 128        slab-major tiles: cs_j = 128, cs_s = p*128
-    // quad = 1 (default, "quad-interleaved" slab-major tiles): inside a slab, columns are grouped by four and the 32-bit
-    // words of the four 128-byte chunks are interleaved, so that 16 consecutive bytes hold word w of columns 4q..4q+3:
-    //   bed + (b>>7)*cs_s + (j>>2)*512 + ((b&127)>>2)*16 + (j&3)*4 + (b&3),  cs_s = p4*128, p4 = p rounded up to 4.
-    // One 128-bit load per lane then feeds four columns with lane = word position, which is what the table lookups of
-    // the sweep need (sweep_ldg.cu) -- no shared-memory staging of the genotype stream.
-    int64_t cs_j = 0, cs_s = 0;
-    int quad = 0;
+    // Quad-interleaved slab-major tiles: the samples are cut into slabs of 512 (128 bytes per column), one slab of all
+    // columns is contiguous, and inside a slab columns are grouped by four with the 32-bit words of their four 128-byte
+    // chunks interleaved, so that 16 consecutive bytes hold word w of columns 4q..4q+3.  Byte b of column j lives at
+    //   bed + (b>>7)*cs_s + (j>>2)*512 + ((b&127)>>2)*16 + (j&3)*4 + (b&3),  cs_s = p4*128.
+    // A sweep stage of 128 columns is then one contiguous 16 KB bulk copy, and one 128-bit shared-memory load per lane
+    // feeds four columns with lane = word position, which is what the table lookups of the sweeps need (sweep_lut.cu).
+    int64_t cs_s = 0;         // bytes per slab
     int64_t p4 = 0;           // columns allocated per slab (p rounded up to a multiple of 4; padding columns are zero)
     int center = 1, scale = 1, impute = 1;
     int sm_count = 148;
@@ -219,22 +217,18 @@ static inline void geno_require_ready(const ihtb_geno* g) {
 // what kernels see of a genotype handle
 struct GenoView {
     const uint8_t* bed;
-    int64_t cs_j, cs_s, nbytes, stride, n, p;
-    int quad;
+    int64_t cs_s, nbytes, stride, n, p;
     const double* mu;
     const double* sinv;
     const int32_t* nmiss;
     int impute;
 };
 static inline GenoView geno_view(const ihtb_geno* g) {
-    return GenoView{g->bed.p, g->cs_j, g->cs_s, g->nbytes, g->stride, g->n, g->p, g->quad, g->mu.p, g->sinv.p,
-                    g->nmiss.p, g->impute};
+    return GenoView{g->bed.p, g->cs_s, g->nbytes, g->stride, g->n, g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->impute};
 }
-// address of byte b of column j; 32-bit words (4-byte aligned b) are contiguous in every layout
+// address of byte b of column j (ihtb_geno::bed); the 4 bytes of a 32-bit word (4-byte aligned b) are contiguous
 __device__ __forceinline__ const uint8_t* gv_ptr(const GenoView& g, int64_t j, int64_t b) {
-    if (g.quad)
-        return g.bed + (b >> 7) * g.cs_s + (j >> 2) * 512 + ((b & 127) >> 2) * 16 + (j & 3) * 4 + (b & 3);
-    return g.bed + j * g.cs_j + (b >> 7) * g.cs_s + (b & 127);
+    return g.bed + (b >> 7) * g.cs_s + (j >> 2) * 512 + ((b & 127) >> 2) * 16 + (j & 3) * 4 + (b & 3);
 }
 
 namespace ihtb {

@@ -60,7 +60,7 @@ __global__ void k_repack(const uint8_t* __restrict__ staging, int64_t pitch, int
     uint32_t q[4];
     memcpy(q, tmp, 16);
 #pragma unroll
-    for (int k = 0; k < 4; ++k)      // words are the contiguous unit of every layout (gv_ptr)
+    for (int k = 0; k < 4; ++k)
         *reinterpret_cast<uint32_t*>(const_cast<uint8_t*>(gv_ptr(g, j0 + c, 16 * v + 4 * k))) = q[k];
 }
 
@@ -245,7 +245,6 @@ __global__ void k_make_tern(GenoView g, int64_t p4, int64_t tern_slabs, uint32_t
 static void build_tern(ihtb_geno* g, cudaStream_t s) {
     g->tern.release();
     g->tern_slabs = 0;
-    if (!g->quad) return;
     const char* e = getenv("IHTB_TERN");
     if (e && *e == '0') return;
     const int64_t slabs = ceil_div(g->n, 640);
@@ -303,13 +302,8 @@ static ihtb_geno* new_handle(int64_t n, int64_t p, int center, int scale, int im
     g->n = n; g->p = p;
     g->nbytes = (n + 3) / 4;
     g->stride = ceil_div(g->nbytes, 128) * 128;
-    // HBM layout (common.cuh): quad-interleaved slab-major tiles by default; IHTB_LAYOUT=tiled keeps plain 128-byte
-    // tiles (the round-1 TMA sweep), IHTB_LAYOUT=colmajor PLINK's column-major order (padded stride, debug only)
-    const char* lay = getenv("IHTB_LAYOUT");
-    g->p4 = (p + 3) / 4 * 4;
-    if (lay && std::string(lay) == "colmajor") { g->cs_j = g->stride; g->cs_s = 128; g->p4 = p; }
-    else if (lay && std::string(lay) == "tiled") { g->cs_j = 128; g->cs_s = g->p * 128; g->p4 = p; }
-    else { g->quad = 1; g->cs_j = 128; g->cs_s = g->p4 * 128; }
+    g->p4 = (p + 3) / 4 * 4;            // quad-interleaved tiles (common.cuh)
+    g->cs_s = g->p4 * 128;
     g->center = center; g->scale = scale; g->impute = impute;
     try {
         g->bed.alloc((size_t)(g->p4 * g->stride));

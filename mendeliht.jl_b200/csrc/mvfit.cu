@@ -408,7 +408,7 @@ struct ihtb_mvfit {
         IHTB_LAUNCH(k_mv_means, 1, 32, 0, s, d_scal.p, r, n, d_vbar.p);
         IHTB_CUDA(cudaMemcpyAsync(h_scal.p, d_scal.p, nv * sizeof(double), cudaMemcpyDeviceToHost, s));
         IHTB_CUDA(cudaEventRecord(ev0, s));
-        const bool l2mode = cfg.sweep_mode == IHTB_SWEEP_PAIR && g->cs_j == 128;
+        const bool l2mode = cfg.sweep_mode == IHTB_SWEEP_PAIR;
         if (l2mode && d_l2.n < (size_t)r) { d_l2.alloc((size_t)r); h_l2.alloc((size_t)r); }
         sweep_xt_v_with_means(g, d_R1.p, d_vbar.p, r, d_dfa.p, cfg.sweep_mode, s, sweep_scratch, nullptr,
                               l2mode ? d_l2.p : nullptr);
@@ -489,7 +489,7 @@ struct ihtb_mvfit {
     std::vector<int64_t> local_candidate_cols(double eta) {
         upload(d_bounds.p, bounds.data(), (size_t)r);
         topk_candidates_blocked(tk, d_dfa.p, d_b0d.p,
-                                (cfg.sweep_mode == IHTB_SWEEP_PAIR && g->cs_j == 128) ? g->sgn.p : g->sinv.p, p,
+                                cfg.sweep_mode == IHTB_SWEEP_PAIR ? g->sgn.p : g->sinv.p, p,
                                 d_bounds.p, eta, cfg.k, s);
         IHTB_CUDA(cudaMemcpyAsync(h_sel.p, d_sel.p, (2 + cap) * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
         sync();

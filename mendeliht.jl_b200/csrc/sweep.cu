@@ -8,12 +8,11 @@
 //     out_jt = sinv_j * (A_jt + mu_j * sum_{missing i} u_it)
 // which equals sinv_j * (sum_i gimp_ij v_it - mu_j sum_i v_it) because mean imputation keeps sum_i gimp_ij = n mu_j.
 //
-//  EXACT: FP64 FMA per genotype, slab partials in FP64 (this file, k_sweep_exact).
+//  EXACT: FP64 nibble-indexed lookup tables in shared memory, slab partials in FP64 (sweep_lut64.cu).
 //  FAST : FP32 byte-indexed lookup tables in shared memory (sweep_lut.cu).
 #include "common.cuh"
 #include "pairer.cuh"
 #include "topk.cuh"
-#include <stdlib.h>
 
 namespace ihtb {
 
@@ -24,69 +23,6 @@ void sweep_exact_lut_partials(const ihtb_geno* g, const double* d_v, const doubl
                               int cls = 0);
 void sweep_pair_partials(const ihtb_geno* g, const double* d_v0, const double* d_v1, const double* d_vbar,
                          const float* d_scale, float* d_part, cudaStream_t s);
-
-// tiled layout: table-driven FP64 kernel (sweep_lut64.cu); column-major debug layout or IHTB_EXACT_LEGACY=1: k_sweep_exact
-static bool exact_uses_lut(const ihtb_geno* g) {
-    static const bool legacy = [] { const char* e = getenv("IHTB_EXACT_LEGACY"); return e && *e == '1'; }();
-    return g->cs_j == 128 && !legacy;
-}
-
-constexpr int EX_THREADS = 128;          // one 32-bit word (16 samples) per thread -> 2048 samples per slab
-constexpr int EX_CB = 8;                 // columns per register tile
-constexpr int EX_COLS_PER_CTA = 512;
-
-__global__ void __launch_bounds__(EX_THREADS)
-k_sweep_exact(GenoView gv, const double* __restrict__ v, const double* __restrict__ vbar_p, double* __restrict__ part /*[n_slabs][p]*/) {
-    const double vbar = *vbar_p;
-    __shared__ double red[EX_THREADS / 32][EX_CB];
-    const int64_t p = gv.p, n = gv.n;
-    const int64_t words = gv.stride >> 2;
-    const int64_t slab = blockIdx.y;
-    const int64_t w = slab * EX_THREADS + threadIdx.x;
-    const bool live = w < words;
-    double u[16];
-#pragma unroll
-    for (int s = 0; s < 16; ++s) {
-        int64_t i = 16 * w + s;
-        u[s] = (live && i < n) ? __dsub_rn(v[i], vbar) : 0.0;
-    }
-    const int64_t jbeg = blockIdx.x * (int64_t)EX_COLS_PER_CTA;
-    const int64_t jend = (jbeg + EX_COLS_PER_CTA < p) ? jbeg + EX_COLS_PER_CTA : p;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int64_t j0 = jbeg; j0 < jend; j0 += EX_CB) {
-        uint32_t wd[EX_CB];
-#pragma unroll
-        for (int c = 0; c < EX_CB; ++c) {
-            int64_t j = j0 + c;
-            wd[c] = (live && j < jend) ? *reinterpret_cast<const uint32_t*>(gv_ptr(gv, j, 4 * w)) : 0u;
-        }
-        double acc[EX_CB];
-#pragma unroll
-        for (int c = 0; c < EX_CB; ++c) {
-            double a = 0.0;
-            uint32_t x = wd[c];
-#pragma unroll
-            for (int s = 0; s < 16; ++s) {
-                uint32_t code = (x >> (2 * s)) & 3u;
-                double dos = (code == 2) ? 1.0 : ((code == 3) ? 2.0 : 0.0);
-                a = fma(u[s], dos, a);
-            }
-            acc[c] = warp_sum(a);
-        }
-        __syncthreads();
-        if (lane == 0) {
-#pragma unroll
-            for (int c = 0; c < EX_CB; ++c) red[warp][c] = acc[c];
-        }
-        __syncthreads();
-        if (threadIdx.x < EX_CB && j0 + threadIdx.x < jend) {
-            double t = 0.0;
-#pragma unroll
-            for (int q = 0; q < EX_THREADS / 32; ++q) t += red[q][threadIdx.x];
-            part[slab * p + j0 + threadIdx.x] = t;
-        }
-    }
-}
 
 // out_j = sinv_j * (sum_s part[s][j] + mu_j * (impute ? sum_{i in miss_j} u_i : -vbar * nmiss_j))
 // tf (optional, tf.keyL != NULL): the first stage of the candidate selection that follows a univariate sweep (topk.cuh
@@ -216,7 +152,7 @@ void sweep_xt_v_with_means(const ihtb_geno* g, const double* dV, const double* d
         for (int64_t t = 0; t < m; ++t) {
             const double* v = dV + t * g->n;
             double* out = dOut + t * g->p;
-            if (mode == IHTB_SWEEP_PAIR && g->cs_j == 128 && t + 1 < m) {
+            if (mode == IHTB_SWEEP_PAIR && t + 1 < m) {
                 // two right-hand sides per pass over the matrix (half2 tables); an odd last one takes the FAST path below
                 const int64_t n_slabs = sweep_fast_num_slabs(g);
                 if (sc->part32.n < (size_t)(2 * n_slabs * g->p)) sc->part32.alloc((size_t)(2 * n_slabs * g->p));
@@ -231,19 +167,10 @@ void sweep_xt_v_with_means(const ihtb_geno* g, const double* dV, const double* d
                 ++t;
                 continue;
             }
-            if (mode == IHTB_SWEEP_EXACT && exact_uses_lut(g)) {
+            if (mode == IHTB_SWEEP_EXACT) {
                 const int64_t n_slabs = g->stride / 128;
                 if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
                 sweep_exact_lut_partials(g, v, d_vbar + t, sc->part64.p, s);
-                IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
-                            g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
-                            g->impute, out, (const float*)nullptr, fuse);
-            } else if (mode == IHTB_SWEEP_EXACT) {
-                int64_t words = g->stride >> 2;
-                int64_t n_slabs = ceil_div(words, EX_THREADS);
-                if (sc->part64.n < (size_t)(n_slabs * g->p)) sc->part64.alloc((size_t)(n_slabs * g->p));
-                dim3 grid((unsigned)ceil_div(g->p, EX_COLS_PER_CTA), (unsigned)n_slabs);
-                IHTB_LAUNCH(k_sweep_exact, grid, EX_THREADS, 0, s, geno_view(g), v, d_vbar + t, sc->part64.p);
                 IHTB_LAUNCH((k_sweep_epilogue<double>), (unsigned)ceil_div(g->p, 256), 256, 0, s, sc->part64.p, n_slabs,
                             g->p, g->mu.p, g->sinv.p, g->nmiss.p, g->miss_ptr.p, g->miss_idx.p, v, d_vbar + t,
                             g->impute, out, (const float*)nullptr, fuse);
@@ -299,7 +226,7 @@ bool SweepPairer::sweep(int slot, const ihtb_geno* g, const double* d_v, const d
     const int other = slot ^ 1;
     IHTB_CUDA(cudaEventRecord(ready[slot], s));        // v / vbar of this fit are complete at this point of its stream
     std::unique_lock<std::mutex> lk(mu);
-    if (active >= 2 && !geno_is_dense(g) && g->cs_j == 128) {
+    if (active >= 2 && !geno_is_dense(g)) {
         req[slot] = Req{d_v, d_vbar, d_out, s};
         has[slot] = true;
         if (has[other]) {
@@ -393,62 +320,36 @@ extern "C" int32_t ihtb_sweep_bench(const ihtb_geno* g, int32_t sweep_mode, int3
         SweepScratch sc;
         cudaEvent_t e0, e1;
         IHTB_CUDA(cudaEventCreate(&e0)); IHTB_CUDA(cudaEventCreate(&e1));
+        // milliseconds per call of `launch`, by CUDA events around `reps` calls on s
+        auto time_reps = [&](auto&& launch) {
+            IHTB_CUDA(cudaEventRecord(e0, s));
+            for (int i = 0; i < reps; ++i) launch();
+            IHTB_CUDA(cudaEventRecord(e1, s));
+            IHTB_CUDA(cudaEventSynchronize(e1));
+            float ms = 0.f;
+            IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+            return (double)(ms / reps);
+        };
         for (int i = 0; i < warmup; ++i)
             sweep_xt_v_with_means(g, dV.p, dmean.p, mrhs, dOut.p, sweep_mode, s, &sc, nullptr, nullptr);
         // (a) whole sweep = partial-sum kernel + epilogue
-        IHTB_CUDA(cudaEventRecord(e0, s));
-        for (int i = 0; i < reps; ++i)
+        const double total = time_reps([&] {
             sweep_xt_v_with_means(g, dV.p, dmean.p, mrhs, dOut.p, sweep_mode, s, &sc, nullptr, nullptr);
-        IHTB_CUDA(cudaEventRecord(e1, s));
-        IHTB_CUDA(cudaEventSynchronize(e1));
-        float ms = 0.f;
-        IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-        if (ms_total) *ms_total = ms / reps;
+        });
+        if (ms_total) *ms_total = total;
         // (b) the dominant kernel alone
         if (ms_kernel) {
             *ms_kernel = 0.0;
-            if (geno_is_dense(g)) {
-                IHTB_CUDA(cudaEventRecord(e0, s));
-                for (int i = 0; i < reps; ++i) dense_sweep_kernel_only(g, dV.p, &sc.part64, s);
-                IHTB_CUDA(cudaEventRecord(e1, s));
-                IHTB_CUDA(cudaEventSynchronize(e1));
-                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-                *ms_kernel = ms / reps;
-            } else if (sweep_mode == IHTB_SWEEP_PAIR) {
-                IHTB_CHECK(g->cs_j == 128, IHTB_EUNSUPPORTED, "the pair sweep needs a tiled layout");
-                IHTB_CUDA(cudaEventRecord(e0, s));
-                for (int i = 0; i < reps; ++i)
+            if (geno_is_dense(g))
+                *ms_kernel = time_reps([&] { dense_sweep_kernel_only(g, dV.p, &sc.part64, s); });
+            else if (sweep_mode == IHTB_SWEEP_PAIR)
+                *ms_kernel = time_reps([&] {
                     sweep_pair_partials(g, dV.p, dV.p + g->n, dmean.p, sc.scale.p, sc.part32.p, s);
-                IHTB_CUDA(cudaEventRecord(e1, s));
-                IHTB_CUDA(cudaEventSynchronize(e1));
-                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-                *ms_kernel = ms / reps;
-            } else if (sweep_mode == IHTB_SWEEP_FAST) {
-                IHTB_CUDA(cudaEventRecord(e0, s));
-                for (int i = 0; i < reps; ++i) sweep_fast_kernel_only(g, dV.p, dmean.p, sc.part32.p, s);
-                IHTB_CUDA(cudaEventRecord(e1, s));
-                IHTB_CUDA(cudaEventSynchronize(e1));
-                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-                *ms_kernel = ms / reps;
-            } else if (exact_uses_lut(g)) {
-                IHTB_CUDA(cudaEventRecord(e0, s));
-                for (int i = 0; i < reps; ++i) sweep_exact_lut_partials(g, dV.p, dmean.p, sc.part64.p, s);
-                IHTB_CUDA(cudaEventRecord(e1, s));
-                IHTB_CUDA(cudaEventSynchronize(e1));
-                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-                *ms_kernel = ms / reps;
-            } else {
-                int64_t words = g->stride >> 2;
-                int64_t n_slabs = ceil_div(words, EX_THREADS);
-                dim3 grid((unsigned)ceil_div(g->p, EX_COLS_PER_CTA), (unsigned)n_slabs);
-                IHTB_CUDA(cudaEventRecord(e0, s));
-                for (int i = 0; i < reps; ++i)
-                    IHTB_LAUNCH(k_sweep_exact, grid, EX_THREADS, 0, s, geno_view(g), dV.p, dmean.p, sc.part64.p);
-                IHTB_CUDA(cudaEventRecord(e1, s));
-                IHTB_CUDA(cudaEventSynchronize(e1));
-                IHTB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-                *ms_kernel = ms / reps;
-            }
+                });
+            else if (sweep_mode == IHTB_SWEEP_FAST)
+                *ms_kernel = time_reps([&] { sweep_fast_kernel_only(g, dV.p, dmean.p, sc.part32.p, s); });
+            else
+                *ms_kernel = time_reps([&] { sweep_exact_lut_partials(g, dV.p, dmean.p, sc.part64.p, s); });
         }
         cudaEventDestroy(e0); cudaEventDestroy(e1);
         cudaStreamDestroy(s);
@@ -460,57 +361,6 @@ extern "C" int32_t ihtb_sweep_bench(const ihtb_geno* g, int32_t sweep_mode, int3
 // With the four possible standardised values of a column, sum x, sum x^2 and sum x*y over the training samples follow
 // from these sums for v = w and v = w.*y, so the univariate regressions need two exact passes over the matrix.
 namespace ihtb {
-
-__global__ void __launch_bounds__(EX_THREADS)
-k_sweep_class_exact(GenoView gv, const double* __restrict__ v, double* __restrict__ part1, double* __restrict__ part2) {
-    __shared__ double red[EX_THREADS / 32][2 * EX_CB];
-    const int64_t p = gv.p, n = gv.n;
-    const int64_t words = gv.stride >> 2;
-    const int64_t slab = blockIdx.y;
-    const int64_t w = slab * EX_THREADS + threadIdx.x;
-    const bool live = w < words;
-    double u[16];
-#pragma unroll
-    for (int s = 0; s < 16; ++s) {
-        int64_t i = 16 * w + s;
-        u[s] = (live && i < n) ? v[i] : 0.0;
-    }
-    const int64_t jbeg = blockIdx.x * (int64_t)EX_COLS_PER_CTA;
-    const int64_t jend = (jbeg + EX_COLS_PER_CTA < p) ? jbeg + EX_COLS_PER_CTA : p;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int64_t j0 = jbeg; j0 < jend; j0 += EX_CB) {
-        double a1[EX_CB], a2[EX_CB];
-#pragma unroll
-        for (int c = 0; c < EX_CB; ++c) {
-            int64_t j = j0 + c;
-            uint32_t x = (live && j < jend) ? *reinterpret_cast<const uint32_t*>(gv_ptr(gv, j, 4 * w)) : 0u;
-            double s1 = 0.0, s2 = 0.0;
-#pragma unroll
-            for (int s = 0; s < 16; ++s) {
-                uint32_t code = (x >> (2 * s)) & 3u;
-                s1 += (code == 2) ? u[s] : 0.0;
-                s2 += (code == 3) ? u[s] : 0.0;
-            }
-            a1[c] = warp_sum(s1);
-            a2[c] = warp_sum(s2);
-        }
-        __syncthreads();
-        if (lane == 0) {
-#pragma unroll
-            for (int c = 0; c < EX_CB; ++c) { red[warp][c] = a1[c]; red[warp][EX_CB + c] = a2[c]; }
-        }
-        __syncthreads();
-        if (threadIdx.x < 2 * EX_CB) {
-            int c = threadIdx.x % EX_CB;
-            if (j0 + c < jend) {
-                double t = 0.0;
-#pragma unroll
-                for (int q = 0; q < EX_THREADS / 32; ++q) t += red[q][threadIdx.x];
-                (threadIdx.x < EX_CB ? part1 : part2)[slab * p + j0 + c] = t;
-            }
-        }
-    }
-}
 
 __global__ void k_class_epilogue(const double* __restrict__ part1, const double* __restrict__ part2, int64_t n_slabs,
                                  int64_t p, const int64_t* __restrict__ miss_ptr, const int32_t* __restrict__ miss_idx,
@@ -527,27 +377,14 @@ __global__ void k_class_epilogue(const double* __restrict__ part1, const double*
 void sweep_class_sums(const ihtb_geno* g, const double* d_v, double* d_w1, double* d_w2, double* d_wm, cudaStream_t s,
                       void* scratch_any) {
     SweepScratch* sc = reinterpret_cast<SweepScratch*>(scratch_any);
-    if (exact_uses_lut(g)) {
-        // table-driven FP64 passes (sweep_lut64.cu) with the indicator maps instead of the dosage: 2 x 3.3 ms at
-        // n = 50k, p = 500k against 10.4 ms for the decode-and-select kernel below
-        const int64_t ns = g->stride / 128;
-        if (sc->part64.n < (size_t)(2 * ns * g->p)) sc->part64.alloc((size_t)(2 * ns * g->p));
-        double* q1 = sc->part64.p;
-        double* q2 = sc->part64.p + ns * g->p;
-        sweep_exact_lut_partials(g, d_v, nullptr, q1, s, 1);
-        sweep_exact_lut_partials(g, d_v, nullptr, q2, s, 2);
-        IHTB_LAUNCH(k_class_epilogue, (unsigned)ceil_div(g->p, 256), 256, 0, s, q1, q2, ns, g->p, g->miss_ptr.p,
-                    g->miss_idx.p, d_v, d_w1, d_w2, d_wm);
-        return;
-    }
-    int64_t words = g->stride >> 2;
-    int64_t n_slabs = ceil_div(words, EX_THREADS);
-    if (sc->part64.n < (size_t)(2 * n_slabs * g->p)) sc->part64.alloc((size_t)(2 * n_slabs * g->p));
-    double* p1 = sc->part64.p;
-    double* p2 = sc->part64.p + n_slabs * g->p;
-    dim3 grid((unsigned)ceil_div(g->p, EX_COLS_PER_CTA), (unsigned)n_slabs);
-    IHTB_LAUNCH(k_sweep_class_exact, grid, EX_THREADS, 0, s, geno_view(g), d_v, p1, p2);
-    IHTB_LAUNCH(k_class_epilogue, (unsigned)ceil_div(g->p, 256), 256, 0, s, p1, p2, n_slabs, g->p, g->miss_ptr.p,
+    // the table-driven FP64 sweep (sweep_lut64.cu) with the indicator maps instead of the dosage, one pass per class
+    const int64_t ns = g->stride / 128;
+    if (sc->part64.n < (size_t)(2 * ns * g->p)) sc->part64.alloc((size_t)(2 * ns * g->p));
+    double* q1 = sc->part64.p;
+    double* q2 = sc->part64.p + ns * g->p;
+    sweep_exact_lut_partials(g, d_v, nullptr, q1, s, 1);
+    sweep_exact_lut_partials(g, d_v, nullptr, q2, s, 2);
+    IHTB_LAUNCH(k_class_epilogue, (unsigned)ceil_div(g->p, 256), 256, 0, s, q1, q2, ns, g->p, g->miss_ptr.p,
                 g->miss_idx.p, d_v, d_w1, d_w2, d_wm);
 }
 

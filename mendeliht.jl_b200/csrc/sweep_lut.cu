@@ -74,9 +74,9 @@ __device__ __forceinline__ LutPlan lut_plan(uint32_t base, uint32_t bytes) {
 // (the mbarrier ABA hazard) and the warp would read a slot before it is refilled.  With per-group full barriers a
 // group sees exactly the fills meant for it, in order, while the groups still progress independently.
 //
-// QUAD: quad-interleaved tiles (common.cuh): a stage is 32 quads of 512 bytes, one LDS.128 per lane fetches word
-//       `lane` of four columns (same wavefronts as four LDS.32, a quarter of the instructions).  `p` is then the padded
-//       column count stored per slab and p_out the number of result columns.
+// A stage of the quad-interleaved tiles (common.cuh) is 32 quads of 512 bytes; one LDS.128 per lane fetches word `lane`
+// of four columns (same wavefronts as four LDS.32, a quarter of the instructions).  `p` is the padded column count
+// stored per slab and p_out the number of result columns.
 // H2:   the PAIR sweep -- two right-hand sides per pass.  The table entries are half2 (v0 | v1), so ONE lookup serves
 //       both: per word four half2 lookups added with HADD2, converted to FP32 and reduced across lanes in FP32.
 //       Entries are scaled by a power of two per right-hand side (max |u| <= 2^9: entries <= 2^12, sums of four
@@ -88,9 +88,9 @@ __device__ __forceinline__ LutPlan lut_plan(uint32_t base, uint32_t bytes) {
 // COL:  TERN && !H2 (the default FAST sweep): 4 groups of 4 warps, 32 columns per warp, and each lane walks the 32 words
 //       of ONE column, so its column sum ends in registers and there is no butterfly.  Shared-memory data-pipe
 //       wavefronts per 128-byte chunk: 4 lookups + 1 read-back, against 6 with the shuffles.  See the consumer below.
-template <int CW, int G, bool QUAD, bool H2, bool TERN>
+template <int CW, int G, bool H2, bool TERN>
 __global__ void __launch_bounds__((CW + 1) * 32, 1)
-k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t p, int64_t p_out, int64_t n,
+k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_s, int64_t p, int64_t p_out, int64_t n,
             int64_t n_slabs, const double* __restrict__ v, const double* __restrict__ v1,
             const double* __restrict__ vbar_p, const float* __restrict__ scale_p, float* __restrict__ part,
             uint32_t dyn_bytes) {
@@ -101,9 +101,9 @@ k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t
     constexpr int WPG = CW / G;                      // warps per group
     constexpr int CPW = LUT_STAGE_COLS / WPG;        // columns per warp per unit
     static_assert(G <= LUT_MAX_GROUPS, "barrier block holds LUT_MAX_GROUPS full barriers per stage");
-    static_assert(!QUAD || CPW % 4 == 0, "quad layout: a warp owns whole quads");
+    static_assert(CPW % 4 == 0, "quad layout: a warp owns whole quads");
     static_assert(!H2 || (CW == 16 && CPW == 16), "pair sweep: 512 table builders, 16 columns per warp");
-    static_assert(!TERN || (QUAD && CW == 16), "ternary tiles: quad layout, 512 table builders");
+    static_assert(!TERN || CW == 16, "ternary tiles: 512 table builders");
     static_assert(!COL || CPW == 32, "one column per lane: 32 columns per warp");
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const LutPlan pl = lut_plan(smem_u32(smem_raw), dyn_bytes);
@@ -142,17 +142,9 @@ k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t
                 const int ncols = (int)((p - j0 < LUT_STAGE_COLS) ? (p - j0) : LUT_STAGE_COLS);
                 const uint32_t fullbar = pl.bar_full + 8u * (uint32_t)(grp_of * LUT_MAX_STAGES + st);
                 mbar_wait(pl.bar_empty + 8u * st, ph ^ 1u);
-                const uint8_t* src = bed + j0 * cs_j + slab * cs_s;
-                if (cs_j == 128) {               // slab-major tiles (plain or quad-interleaved): one contiguous copy
-                    if (lane == 0) {
-                        mbar_expect_tx(fullbar, (uint32_t)ncols * 128u);
-                        bulk_g2s(pl.stage(st), src, (uint32_t)ncols * 128u, fullbar);
-                    }
-                } else {                          // column-major layout: one 128-byte copy per column
-                    if (lane == 0) mbar_expect_tx(fullbar, (uint32_t)ncols * 128u);
-                    __syncwarp();
-                    for (int c = lane; c < ncols; c += 32)
-                        bulk_g2s(pl.stage(st) + 128u * c, src + (int64_t)c * cs_j, 128u, fullbar);
+                if (lane == 0) {
+                    mbar_expect_tx(fullbar, (uint32_t)ncols * 128u);
+                    bulk_g2s(pl.stage(st), bed + j0 * 128 + slab * cs_s, (uint32_t)ncols * 128u, fullbar);
                 }
                 if (++st == S) { st = 0; ph ^= 1u; }
                 if (++grp_of == G) grp_of = 0;
@@ -180,7 +172,7 @@ k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t
         const int col = wg * CPW + vidx % CPW;        // column (within a unit) this lane stores
         const bool writer = TERN ? (lane < NACC) : (lane & (LPC - 1)) == 0;
         const uint32_t lqs = TERN ? ((((uint32_t)lane >> 2) & 3u) << 9) : 0u;
-        const uint32_t lane_off = (uint32_t)(wg * CPW) * 128u + (QUAD ? 16u : 4u) * (uint32_t)lane;
+        const uint32_t lane_off = (uint32_t)(wg * CPW) * 128u + 16u * (uint32_t)lane;
         // COL: lane l owns component ci = l & 3 of the warp's quad ql = l >> 2, i.e. column 4 ql + ci = l of the warp, and
         // at step s = 0..31 takes word position w = w0 ^ s, w0 = 8 ci + ql.  In the tiles that word sits at byte
         // 512 ql + 16 w + 4 (ci ^ (w & 3)) = D0 ^ K(s) with K(s) = 16 s + 4 (s & 3) (disjoint bit fields), so with
@@ -249,13 +241,8 @@ k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t
                     uint4 q4 = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
                     for (int c = 0; c < CPW; ++c) {
-                        uint32_t w;
-                        if (QUAD) {
-                            if ((c & 3) == 0) q4 = lds_u128(colbase + ((512u * (c >> 2)) ^ lqs));
-                            w = (c & 3) == 0 ? q4.x : (c & 3) == 1 ? q4.y : (c & 3) == 2 ? q4.z : q4.w;
-                        } else {
-                            w = lds_u32(colbase + 128u * c);
-                        }
+                        if ((c & 3) == 0) q4 = lds_u128(colbase + ((512u * (c >> 2)) ^ lqs));
+                        const uint32_t w = (c & 3) == 0 ? q4.x : (c & 3) == 1 ? q4.y : (c & 3) == 2 ? q4.z : q4.w;
                         if (!H2) {
                             const float t0 = lds_f32(__byte_perm(w, lb[0], 0x7604));
                             const float t1 = lds_f32(__byte_perm(w, lb[1], 0x7614));
@@ -313,39 +300,30 @@ k_sweep_lut(const uint8_t* __restrict__ bed, int64_t cs_j, int64_t cs_s, int64_t
     }
 }
 
-// the FAST / PAIR sweeps stream the ternary copy when the handle has one (the TMEM variant reads the 2-bit tiles)
-bool sweep_tmem_enabled(const ihtb_geno* g);
-bool sweep_uses_tern(const ihtb_geno* g) { return g->tern.p != nullptr && g->quad && !sweep_tmem_enabled(g); }
+// the FAST / PAIR sweeps stream the ternary copy when the handle has one
+bool sweep_uses_tern(const ihtb_geno* g) { return g->tern.p != nullptr; }
 int64_t sweep_fast_num_slabs(const ihtb_geno* g) { return sweep_uses_tern(g) ? g->tern_slabs : g->stride / 128; }
 
-// sweep_tmem.cu: the same sweeps with the genotype stream staged through tensor memory (quad layout only)
-bool sweep_tmem_enabled(const ihtb_geno* g);
-void sweep_tmem_partials(const ihtb_geno* g, const double* d_v, const double* d_vbar, float* d_part, cudaStream_t s);
-void sweep_tmem_pair_partials(const ihtb_geno* g, const double* d_v0, const double* d_v1, const double* d_vbar,
-                              const float* d_scale, float* d_part, cudaStream_t s);
-
-template <bool QUAD, bool H2, bool TERN = false>
+template <bool H2, bool TERN>
 static void launch_lut(const ihtb_geno* g, const double* d_v, const double* d_v1, const double* d_vbar,
                        const float* d_scale, float* d_part, cudaStream_t s) {
     constexpr int G = (TERN && !H2) ? 4 : 2;         // one column per lane: 4 warps cover a 128-column unit
-    ensure_dynamic_smem(k_sweep_lut<16, G, QUAD, H2, TERN>, LUT_SMEM_BYTES);
+    ensure_dynamic_smem(k_sweep_lut<16, G, H2, TERN>, LUT_SMEM_BYTES);
     const int64_t n_slabs = TERN ? g->tern_slabs : g->stride / 128;
     const int64_t n_cblocks = ceil_div(g->p4, LUT_STAGE_COLS);
     int64_t units = n_slabs * n_cblocks;
     int grid = g->sm_count;
     if (units < grid) grid = (int)units;
     IHTB_CHECK(g->p < (int64_t(1) << 31) - 256, IHTB_EDIM, "more than 2^31 SNP columns on one GPU");
-    IHTB_LAUNCH((k_sweep_lut<16, G, QUAD, H2, TERN>), grid, 17 * 32, LUT_SMEM_BYTES, s, TERN ? g->tern.p : g->bed.p, g->cs_j,
-                g->cs_s, g->p4, g->p, g->n, n_slabs, d_v, d_v1, d_vbar, d_scale, d_part, (uint32_t)LUT_SMEM_BYTES);
+    IHTB_LAUNCH((k_sweep_lut<16, G, H2, TERN>), grid, 17 * 32, LUT_SMEM_BYTES, s, TERN ? g->tern.p : g->bed.p, g->cs_s,
+                g->p4, g->p, g->n, n_slabs, d_v, d_v1, d_vbar, d_scale, d_part, (uint32_t)LUT_SMEM_BYTES);
 }
 
 // FAST sweep, one right-hand side: d_part is [n_slabs][p] floats
 void sweep_fast_partials(const ihtb_geno* g, const double* d_v, const double* d_vbar, float* d_part, int64_t* n_slabs_out,
                          cudaStream_t s) {
     if (n_slabs_out) *n_slabs_out = sweep_fast_num_slabs(g);
-    if (sweep_tmem_enabled(g)) { sweep_tmem_partials(g, d_v, d_vbar, d_part, s); return; }
-    if (sweep_uses_tern(g)) launch_lut<true, false, true>(g, d_v, nullptr, d_vbar, nullptr, d_part, s);
-    else if (g->quad) launch_lut<true, false>(g, d_v, nullptr, d_vbar, nullptr, d_part, s);
+    if (sweep_uses_tern(g)) launch_lut<false, true>(g, d_v, nullptr, d_vbar, nullptr, d_part, s);
     else launch_lut<false, false>(g, d_v, nullptr, d_vbar, nullptr, d_part, s);
 }
 
@@ -357,11 +335,8 @@ void sweep_fast_kernel_only(const ihtb_geno* g, const double* d_v, const double*
 // d_part is [2][n_slabs][p] floats of the scaled sums
 void sweep_pair_partials(const ihtb_geno* g, const double* d_v0, const double* d_v1, const double* d_vbar,
                          const float* d_scale, float* d_part, cudaStream_t s) {
-    IHTB_CHECK(g->cs_j == 128, IHTB_EUNSUPPORTED, "the pair sweep needs a tiled layout");
-    if (sweep_tmem_enabled(g)) { sweep_tmem_pair_partials(g, d_v0, d_v1, d_vbar, d_scale, d_part, s); return; }
-    if (sweep_uses_tern(g)) launch_lut<true, true, true>(g, d_v0, d_v1, d_vbar, d_scale, d_part, s);
-    else if (g->quad) launch_lut<true, true>(g, d_v0, d_v1, d_vbar, d_scale, d_part, s);
-    else launch_lut<false, true>(g, d_v0, d_v1, d_vbar, d_scale, d_part, s);
+    if (sweep_uses_tern(g)) launch_lut<true, true>(g, d_v0, d_v1, d_vbar, d_scale, d_part, s);
+    else launch_lut<true, false>(g, d_v0, d_v1, d_vbar, d_scale, d_part, s);
 }
 
 }  // namespace ihtb

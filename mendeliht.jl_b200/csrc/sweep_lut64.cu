@@ -1,9 +1,8 @@
 // EXACT X'v sweep for sm_100a: FP64 lookup tables indexed by NIBBLE (2 genotypes), same TMA pipeline as sweep_lut.cu.
 //
-// The first exact kernel (k_sweep_exact, sweep.cu: shift/compare/select/DFMA per genotype, kept for the column-major
-// debug layout) is issue-bound at 0.6 TB/s.  A byte-indexed FP64 table like the FAST kernel's would need 256 KB per
-// 512-sample slab, so here a table row covers 2 samples: for the 32 words w of a column chunk and the 8 nibbles t of
-// a word
+// A shift/compare/select/DFMA per genotype (the first exact kernel) is issue-bound at 0.6 TB/s.  A byte-indexed FP64
+// table like the FAST kernel's would need 256 KB per 512-sample slab, so here a table row covers 2 samples: for the 32
+// words w of a column chunk and the 8 nibbles t of a word
 //     T[t][value][w] = dosage(value & 3) * u[512*slab + 16*w + 2*t] + dosage(value >> 2) * u[512*slab + 16*w + 2*t + 1],
 // u = v - mean(v) in FP64: 8 * 16 * 32 doubles = 32 KB.  Lane w owns word w of a column chunk; the 32 lanes of one
 // LDS.64 read 32 consecutive doubles of a row whatever the data are (2 wavefronts, the minimum for 256 bytes).  Rows
@@ -51,11 +50,6 @@ __device__ __forceinline__ double lds_f64(uint32_t addr) {
     asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
     return v;
 }
-__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
 __device__ __forceinline__ void sts_f64(uint32_t addr, double v) {
     asm volatile("st.shared.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
 }
@@ -98,10 +92,9 @@ __device__ __forceinline__ uint4 lds_u128(uint32_t addr) {
     return v;
 }
 
-// QUAD: quad-interleaved tiles (common.cuh) -- a stage holds 32 quads of 512 bytes, 16 bytes per (quad, word): one
-// LDS.128 per lane fetches word `lane` of four columns (same wavefront count as four LDS.32 on plain tiles).
-// p is the number of columns stored per slab (p4 for QUAD); p_out the number of result columns.
-template <bool QUAD>
+// Quad-interleaved tiles (common.cuh): a stage holds 32 quads of 512 bytes, 16 bytes per (quad, word), so one LDS.128
+// per lane fetches word `lane` of four columns (same wavefront count as four LDS.32).
+// p is the number of columns stored per slab (p4); p_out the number of result columns.
 __global__ void __launch_bounds__((X_CW + 1) * 32, 1)
 k_sweep_lut64(const uint8_t* __restrict__ bed, int64_t cs_s, int64_t p, int64_t p_out, int64_t n, int64_t n_slabs,
               const double* __restrict__ v, const double* __restrict__ vbar_p, double* __restrict__ part, int cls) {
@@ -165,8 +158,7 @@ k_sweep_lut64(const uint8_t* __restrict__ bed, int64_t cs_s, int64_t p, int64_t 
         constexpr int LPC = 32 / CPW;
         const int col = wg * CPW + lane / LPC;
         const bool writer = (lane & (LPC - 1)) == 0;
-        const uint32_t lane_off = QUAD ? (uint32_t)(wg * CPW) * 128u + 16u * (uint32_t)lane
-                                       : (uint32_t)(wg * CPW) * 128u + 4u * (uint32_t)lane;
+        const uint32_t lane_off = (uint32_t)(wg * CPW) * 128u + 16u * (uint32_t)lane;
         int st = grp % S, ip = grp % period; uint32_t ph = (uint32_t)((grp / period) & 1);
         const uint32_t my_full = bar_full + 8u * (uint32_t)(grp * S);
         int i_next = grp;
@@ -187,13 +179,8 @@ k_sweep_lut64(const uint8_t* __restrict__ bed, int64_t cs_s, int64_t p, int64_t 
                 uint4 q4 = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
                 for (int c = 0; c < CPW; ++c) {
-                    uint32_t w;
-                    if (QUAD) {
-                        if ((c & 3) == 0) q4 = lds_u128(colbase + 512u * (c >> 2));
-                        w = (c & 3) == 0 ? q4.x : (c & 3) == 1 ? q4.y : (c & 3) == 2 ? q4.z : q4.w;
-                    } else {
-                        w = lds_u32(colbase + 128u * c);
-                    }
+                    if ((c & 3) == 0) q4 = lds_u128(colbase + 512u * (c >> 2));
+                    const uint32_t w = (c & 3) == 0 ? q4.x : (c & 3) == 1 ? q4.y : (c & 3) == 2 ? q4.z : q4.w;
                     const double d0 = lds_f64(lb[0] | ((w << 8) & 0xF00u));
                     const double d1 = lds_f64(lb[1] | ((w << 4) & 0xF00u));
                     const double d2 = lds_f64(lb[2] | (w & 0xF00u));
@@ -232,24 +219,17 @@ k_sweep_lut64(const uint8_t* __restrict__ bed, int64_t cs_s, int64_t p, int64_t 
 
 }  // namespace
 
-// tiled layouts only (cs_j == 128, plain or quad-interleaved); d_part is [stride/128][p] doubles
+// d_part is [stride/128][p] doubles
 void sweep_exact_lut_partials(const ihtb_geno* g, const double* d_v, const double* d_vbar, double* d_part, cudaStream_t s,
                               int cls) {
-    IHTB_CHECK(g->cs_j == 128, IHTB_EINVAL, "the table-driven exact sweep needs a tiled layout");
     IHTB_CHECK(g->p < (int64_t(1) << 31) - 256, IHTB_EDIM, "more than 2^31 SNP columns on one GPU");
     const int64_t n_slabs = g->stride / 128;
     const int64_t units = n_slabs * ceil_div(g->p4, X_STAGE_COLS);
     int grid = g->sm_count;
     if (units < grid) grid = (int)units;
-    if (g->quad) {
-        ensure_dynamic_smem(k_sweep_lut64<true>, X_SMEM_BYTES);
-        IHTB_LAUNCH(k_sweep_lut64<true>, grid, (X_CW + 1) * 32, X_SMEM_BYTES, s, g->bed.p, g->cs_s, g->p4, g->p, g->n,
-                    n_slabs, d_v, d_vbar, d_part, cls);
-    } else {
-        ensure_dynamic_smem(k_sweep_lut64<false>, X_SMEM_BYTES);
-        IHTB_LAUNCH(k_sweep_lut64<false>, grid, (X_CW + 1) * 32, X_SMEM_BYTES, s, g->bed.p, g->cs_s, g->p, g->p, g->n,
-                    n_slabs, d_v, d_vbar, d_part, cls);
-    }
+    ensure_dynamic_smem(k_sweep_lut64, X_SMEM_BYTES);
+    IHTB_LAUNCH(k_sweep_lut64, grid, (X_CW + 1) * 32, X_SMEM_BYTES, s, g->bed.p, g->cs_s, g->p4, g->p, g->n, n_slabs, d_v,
+                d_vbar, d_part, cls);
 }
 
 }  // namespace ihtb

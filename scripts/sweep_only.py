@@ -1,6 +1,6 @@
 """Runs the X'r sweep alone on a device-generated matrix (for ncu captures and quick kernel timing).
 usage: sweep_only.py [n p reps mode]   mode 0 = FAST, 1 = EXACT, 2 = PAIR (two right-hand sides per pass)
-env:   IHTB_LAYOUT=quad|tiled|colmajor, IHTB_TERN=0|1 (ternary copy of the tiles: default on when memory allows)"""
+env:   IHTB_TERN=0|1 (ternary copy of the tiles: default on when memory allows)"""
 import ctypes as C
 import json
 import os
@@ -18,7 +18,7 @@ mk, mt = C.c_double(0), C.c_double(0)
 m._lib.check(m.load().ihtb_sweep_bench(g._h, mode, 2, reps, C.byref(mk), C.byref(mt)))
 b = p * ((n + 3) // 4) + 8 * n + 24 * p
 rhs = 2 if mode == 2 else 1
-print(json.dumps({"n": n, "p": p, "mode": ["FAST", "EXACT", "PAIR"][mode], "layout": os.environ.get("IHTB_LAYOUT", "quad"),
+print(json.dumps({"n": n, "p": p, "mode": ["FAST", "EXACT", "PAIR"][mode],
                   "ternary": g.sweep_stream_bytes()[1], "streamed_GBs": round((g.sweep_stream_bytes()[0] + 8 * n + 24 * p) / mk.value / 1e6, 1)
                   if mode != 1 else None, "rhs_per_pass": rhs,
                   "kernel_ms": round(mk.value, 4), "total_ms": round(mt.value, 4),

@@ -10,22 +10,11 @@ import mendeliht_jl_b200 as m
 from mendeliht_jl_b200 import synth
 from oracle import snp
 
-LAYOUTS = ["quad", "tiled", "colmajor"]     # quad = the default quad-interleaved tiles (common.cuh)
 
-
-def _make(bed, n, layout):
-    os.environ["IHTB_LAYOUT"] = layout
-    try:
-        return m.B200SnpLinAlg.from_bed_columns(bed, n)
-    finally:
-        os.environ.pop("IHTB_LAYOUT", None)
-
-
-@pytest.mark.parametrize("layout", LAYOUTS)
 @pytest.mark.parametrize("n,p,miss", [(1000, 257, 0.0), (1003, 300, 0.02), (515, 64, 0.3), (7, 5, 0.0), (2049, 130, 0.001)])
-def test_stats_decode_packed_bit_exact(layout, n, p, miss):
+def test_stats_decode_packed_bit_exact(n, p, miss):
     bed = synth.packed_columns(11, n, np.arange(p), miss)
-    g = _make(bed, n, layout)
+    g = m.B200SnpLinAlg.from_bed_columns(bed, n)
     o = snp.SnpLinAlgOracle(bed, n)
     mu, sinv, nm = g.stats()
     assert np.array_equal(nm, o.nmiss)
@@ -36,22 +25,16 @@ def test_stats_decode_packed_bit_exact(layout, n, p, miss):
     assert np.array_equal(g.packed(), bed)
 
 
-@pytest.mark.parametrize("layout", LAYOUTS)
-def test_device_generator_matches_numpy_twin(layout):
-    os.environ["IHTB_LAYOUT"] = layout
-    try:
-        for n, p, miss, j0 in [(1003, 200, 0.0, 0), (2500, 150, 0.01, 1000)]:
-            g = m.B200SnpLinAlg.synthetic(n, p, 2024, miss, j0)
-            assert np.array_equal(g.packed(), synth.packed_columns(2024, n, np.arange(j0, j0 + p), miss))
-    finally:
-        os.environ.pop("IHTB_LAYOUT", None)
+def test_device_generator_matches_numpy_twin():
+    for n, p, miss, j0 in [(1003, 200, 0.0, 0), (2500, 150, 0.01, 1000)]:
+        g = m.B200SnpLinAlg.synthetic(n, p, 2024, miss, j0)
+        assert np.array_equal(g.packed(), synth.packed_columns(2024, n, np.arange(j0, j0 + p), miss))
 
 
-@pytest.mark.parametrize("layout", LAYOUTS)
 @pytest.mark.parametrize("n,p,miss", [(1000, 300, 0.0), (1003, 513, 0.01), (4099, 260, 0.0), (600, 129, 0.2)])
-def test_xt_v_exact_and_fast(layout, n, p, miss):
+def test_xt_v_exact_and_fast(n, p, miss):
     bed = synth.packed_columns(5, n, np.arange(p), miss)
-    g = _make(bed, n, layout)
+    g = m.B200SnpLinAlg.from_bed_columns(bed, n)
     o = snp.SnpLinAlgOracle(bed, n)
     rng = np.random.default_rng(0)
     v = rng.normal(size=n) + 0.3
@@ -72,20 +55,19 @@ def test_xt_v_exact_and_fast(layout, n, p, miss):
     np.testing.assert_allclose(b, 2 * a, rtol=0, atol=1e-10 * scale)    # centring kills the constant
     # pair sweep (two right-hand sides per pass, half2 tables): proven bound 2^-8 * ||v - mean||_1 * sinv per entry;
     # right-hand sides of very different magnitude exercise the per-vector power-of-two scaling
-    if layout != "colmajor":
-        V5 = rng.normal(size=(n, 5)) * np.array([1.0, 1e-6, 3e4, 0.02, 7.0]) + np.array([0.0, 1.0, -5.0, 0.0, 2.0])
-        got, want = g.xt_v(V5, m.SWEEP_PAIR), o.xt_v(V5)
-        # the bound the fits use: 3.1 * 2^-11 * ||u||_2 * sinv_j * max(sqrt(sum_i g_ij^2), 1)  (Cauchy-Schwarz on the
-        # absolute dot product every FP16 rounding is relative to); the last, odd vector takes the FP32 tables
-        gn = np.maximum(np.sqrt((np.where(np.isnan(snp.dosages(bed, n)), 0.0, snp.dosages(bed, n)) ** 2).sum(axis=0)), 1.0)
-        for t in range(5):
-            u = V5[:, t] - V5[:, t].mean()
-            bnd = (3.1 * 2.0 ** -11 if t < 4 else 2.0 ** -20) * np.sqrt((u ** 2).sum()) * o.sigma_inv * gn
-            assert np.all(np.abs(got[:, t] - want[:, t]) <= bnd + 1e-12 * np.abs(want[:, t]).max()), t
-            assert np.all(np.abs(got[:, t] - want[:, t]) <= (2.0 ** -8) * np.abs(u).sum() * o.sigma_inv + 1e-12 * np.abs(want[:, t]).max())
-        assert np.array_equal(g.xt_v(V5[:, :1], m.SWEEP_PAIR), g.xt_v(V5[:, :1], m.SWEEP_FAST))   # odd one out: FAST
-        zero = np.zeros((n, 2)); zero[:, 1] = 3.0                      # constant vectors: u = 0, scale falls back to 1
-        assert np.all(g.xt_v(zero, m.SWEEP_PAIR) == 0.0)
+    V5 = rng.normal(size=(n, 5)) * np.array([1.0, 1e-6, 3e4, 0.02, 7.0]) + np.array([0.0, 1.0, -5.0, 0.0, 2.0])
+    got, want = g.xt_v(V5, m.SWEEP_PAIR), o.xt_v(V5)
+    # the bound the fits use: 3.1 * 2^-11 * ||u||_2 * sinv_j * max(sqrt(sum_i g_ij^2), 1)  (Cauchy-Schwarz on the
+    # absolute dot product every FP16 rounding is relative to); the last, odd vector takes the FP32 tables
+    gn = np.maximum(np.sqrt((np.where(np.isnan(snp.dosages(bed, n)), 0.0, snp.dosages(bed, n)) ** 2).sum(axis=0)), 1.0)
+    for t in range(5):
+        u = V5[:, t] - V5[:, t].mean()
+        bnd = (3.1 * 2.0 ** -11 if t < 4 else 2.0 ** -20) * np.sqrt((u ** 2).sum()) * o.sigma_inv * gn
+        assert np.all(np.abs(got[:, t] - want[:, t]) <= bnd + 1e-12 * np.abs(want[:, t]).max()), t
+        assert np.all(np.abs(got[:, t] - want[:, t]) <= (2.0 ** -8) * np.abs(u).sum() * o.sigma_inv + 1e-12 * np.abs(want[:, t]).max())
+    assert np.array_equal(g.xt_v(V5[:, :1], m.SWEEP_PAIR), g.xt_v(V5[:, :1], m.SWEEP_FAST))   # odd one out: FAST
+    zero = np.zeros((n, 2)); zero[:, 1] = 3.0                      # constant vectors: u = 0, scale falls back to 1
+    assert np.all(g.xt_v(zero, m.SWEEP_PAIR) == 0.0)
 
 
 @pytest.mark.parametrize("n,p,miss", [(1003, 513, 0.01), (640, 9, 0.0), (641, 130, 0.3), (3200, 257, 0.0), (50, 4, 0.0),
@@ -128,32 +110,10 @@ def test_ternary_copy_sweeps(n, p, miss):
         g.close()
 
 
-def test_tensor_memory_sweep_matches_stage_ring():
-    """IHTB_SWEEP_TMEM=1: the genotype stream staged through tensor memory (tcgen05.cp / tcgen05.ld, sweep_tmem.cu).
-    Same tables, same butterfly, same partial sums per slab: results identical to the default kernel, FAST and PAIR,
-    including ragged n and a column count that is not a multiple of the 256-column unit."""
-    for n, p, miss in [(1003, 513, 0.01), (5000, 3001, 0.0), (600, 7, 0.2)]:
-        bed = synth.packed_columns(5, n, np.arange(p), miss)
-        os.environ["IHTB_TERN"] = "0"           # both kernels on the 2-bit tiles (the TMEM variant has no ternary form)
-        try:
-            g = m.B200SnpLinAlg.from_bed_columns(bed, n)
-        finally:
-            os.environ.pop("IHTB_TERN", None)
-        V = np.random.default_rng(2).normal(size=(n, 2)) * np.array([1.0, 30.0]) + 0.3
-        want_f, want_p = g.xt_v(V[:, 0], m.SWEEP_FAST), g.xt_v(V, m.SWEEP_PAIR)
-        os.environ["IHTB_SWEEP_TMEM"] = "1"
-        try:
-            got_f, got_p = g.xt_v(V[:, 0], m.SWEEP_FAST), g.xt_v(V, m.SWEEP_PAIR)
-        finally:
-            os.environ.pop("IHTB_SWEEP_TMEM", None)
-        assert np.array_equal(got_f, want_f) and np.array_equal(got_p, want_p)
-
-
-@pytest.mark.parametrize("layout", LAYOUTS)
-def test_x_support_bit_exact(layout):
+def test_x_support_bit_exact():
     n, p = 1003, 400
     bed = synth.packed_columns(9, n, np.arange(p), 0.01)
-    g = _make(bed, n, layout)
+    g = m.B200SnpLinAlg.from_bed_columns(bed, n)
     o = snp.SnpLinAlgOracle(bed, n)
     rng = np.random.default_rng(1)
     idx = np.sort(rng.permutation(p)[:37])
