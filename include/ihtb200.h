@@ -160,6 +160,8 @@ int32_t ihtb_geno_destroy(ihtb_geno* g);
  * ihtb_geno_decode the stored values, ihtb_geno_sweep_stream_bytes n*p*sizeof(T) with ternary = 0 (2*n*p for
  * IHTB_DENSE_FIX16 below); ihtb_geno_packed,
  * counts, maf, ternary_tiles, gather_bench and set_offset return IHTB_EUNSUPPORTED and load_columns IHTB_EINVAL.
+ * BGEN files load into FIX16 / F64 handles through ihtb_geno_load_bgen_columns, over all of a file's samples or over a
+ * chosen subset in a chosen row order (ihtb_geno_select_bgen_samples; n is then the number of kept samples).
  * Not supported on a DENSE handle (IHTB_EUNSUPPORTED): multivariate fits, SNP-sharded fits, multi-device handles. */
 enum { IHTB_DENSE_F64 = 0, IHTB_DENSE_F32 = 1, IHTB_DENSE_FIX16 = 2 };
 /* dtype IHTB_DENSE_F64 or IHTB_DENSE_F32 (IHTB_DENSE_FIX16 needs a denominator: ihtb_geno_create_dosage16) */
@@ -194,15 +196,25 @@ int32_t ihtb_geno_create_dosage16_empty(int64_t n, int64_t p, int32_t denominato
  * (2 D - code).  FIX16 handles store the code and need D == the handle's denominator (so B <= 15); F64 handles store
  * code / D (IEEE FP64 division, any B).  A missing sample is stored as IHTB_DOSAGE16_MISSING / NaN, so it needs
  * standardize = 1 at ihtb_geno_finalize, as for the other loaders.  The blocks are staged through two pinned buffers
- * and decoded on the device (one CTA per block).  Errors name the LOWEST failing block and the reason:
- *   IHTB_EDIM         block N != n
- *   IHTB_EUNSUPPORTED K != 2, or ploidy != 2 on a non-missing sample
+ * and decoded on the device (one CTA per block).  After ihtb_geno_select_bgen_samples (below) every block holds n_file
+ * samples and row i is decoded from file sample rows[i]; only kept samples are read and checked (missing flag, ploidy,
+ * a + b <= D), and errors name file sample indices.  Errors name the LOWEST failing block and the reason:
+ *   IHTB_EDIM         block N != n (with a selection: != n_file)
+ *   IHTB_EUNSUPPORTED K != 2, or ploidy != 2 on a non-missing (kept) sample
  *   IHTB_EINVAL       B = 0, B > 32, 2^B - 1 != the FIX16 denominator, phased flag not 0 / 1, a block shorter than its
  *                     header + ceil(2 N B / 8) bytes; an F32 handle, allele not 1 / 2, decreasing offsets
  *   IHTB_EDOMAIN      unphased a + b > D
  * After an error the contents of the columns of this call are unspecified (load them again or destroy the handle). */
 int32_t ihtb_geno_load_bgen_columns(ihtb_geno* g, const uint8_t* blocks, const int64_t* offsets, int64_t j_first,
                                     int64_t ncols, int32_t allele);
+/* Keep a subset of a BGEN file's samples, in a chosen order, when loading into an unfinalized handle:
+ * row i of the handle is file sample rows[i], for i in [0, n).  rows: n distinct values in [0, n_file), any order.
+ * Allowed only on an unfinalized IHTB_DENSE_FIX16 or IHTB_DENSE_F64 handle before its first
+ * ihtb_geno_load_bgen_columns call, so every column of a handle comes from one selection; IHTB_EINVAL otherwise (PLINK,
+ * F32 or finalized handle, BGEN columns already loaded), and for n > n_file, n_file > 2^32 - 1, a row out of range
+ * (naming its position and value) or a repeated row (naming both positions).  The map is held on the device as 32-bit
+ * indices with the staging buffers, uploaded once, and released at ihtb_geno_finalize.  Rows n..ld-1 stay zero. */
+int32_t ihtb_geno_select_bgen_samples(ihtb_geno* g, const int64_t* rows, int64_t n_file);
 /* Host staging batch of ihtb_geno_load_bgen_columns in bytes (whole blocks, at least one per batch; default 64 MiB,
  * restored by bytes <= 0).  Process-wide; a tuning and test knob. */
 int32_t ihtb_bgen_set_batch_bytes(int64_t bytes);

@@ -308,18 +308,31 @@ class B200DenseLinAlg:
         return obj
 
     @classmethod
-    def from_bgen(cls, paths, standardize: bool = False, allele: int = 2, storage: str = "auto") -> "B200DenseLinAlg":
+    def from_bgen(cls, paths, standardize: bool = False, allele: int = 2, storage: str = "auto", samples=None,
+                  sample_file=None, variants=None) -> "B200DenseLinAlg":
         """Dosages of BGEN 1.2 files (layout 2, uncompressed or zlib; biallelic diploid variants).  `paths`: one file or
         a list (e.g. one per chromosome) over the same samples -- N must match, and so must the sample IDs where files
         carry them -- whose variants become the columns in the order given.  A probability stored as a B-bit integer
         makes the dosage of `allele` (2, the default: copies of the second allele, what a PLINK handle counts; or 1)
         exactly code / (2^B - 1); the host inflates the blocks (thread pool, ~64 MB batches) and the device decodes them
         (ihtb_geno_load_bgen_columns).  storage="auto": 16-bit codes with denominator 2^B - 1 (as `from_dosages`) when
-        the first variant has B <= 15, Float64 otherwise; "fix16" / "f64" force one (a FIX16 handle needs the same B in
-        every variant).  Missing samples need standardize=True, as NaN does for `from_array`.  The handle equals
-        `from_dosages(codes / D, D, standardize)` (FIX16) or `from_array(codes / D, standardize)` bit for bit
-        (bgen.dosage_codes is the host twin), and carries `.variants` (bgen.BgenVariant per column) and `.samples`
-        (sample IDs, or None when no file stores them)."""
+        the first kept variant has B <= 15, Float64 otherwise; "fix16" / "f64" force one (a FIX16 handle needs the same
+        B in every kept variant).  Missing samples need standardize=True, as NaN does for `from_array`.
+
+        samples: None keeps every sample in file order; a sequence of ints (0-based file positions) or of strings (IDs,
+        looked up in `sample_file` when given, else in the IDs the files embed) keeps those samples, in that order: it
+        is the row order, so phenotypes follow it.  sample_file: an Oxford .sample file (bgen.read_sample_file) with N
+        samples, identical to the embedded IDs where the files carry them.  variants: None keeps every variant; a
+        boolean mask over the concatenated variants, strictly increasing indices into them, or a callable
+        BgenVariant -> bool.  Only kept variants are inflated and loaded, and only kept samples are decoded and checked
+        on the device (ihtb_geno_select_bgen_samples).  Every argument error raises ValueError before the device is
+        touched; an empty selection raises DimensionMismatch.
+
+        With codes [N, p] of the files (bgen.dosage_codes is the host twin), rows the kept samples and cols the kept
+        variants, the handle equals `from_dosages(codes[rows][:, cols] / D, D, standardize)` (FIX16) or
+        `from_array(codes[rows][:, cols] / D, standardize)` bit for bit, so standardization uses the kept samples only.
+        It carries `.variants` (bgen.BgenVariant per kept column) and `.samples` (kept sample IDs in row order, or None
+        when no file and no sample_file stores them)."""
         from . import bgen as _bgen
         if isinstance(paths, (str, bytes, os.PathLike)):
             paths = [paths]
@@ -335,47 +348,73 @@ class B200DenseLinAlg:
             for q in paths:
                 files.append(_bgen.BgenFile(q))
             n = files[0].n
-            samples, samples_from = None, None
+            ids, ids_from = None, None
             for f in files:
                 if f.n != n:
                     raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"{f.path} holds {f.n} samples, {files[0].path} {n}")
                 if f.samples is not None:
-                    if samples is None:
-                        samples, samples_from = f.samples, f.path
-                    elif f.samples != samples:
-                        raise ValueError(f"{f.path}: sample identifiers differ from those of {samples_from}")
+                    if ids is None:
+                        ids, ids_from = f.samples, f.path
+                    elif f.samples != ids:
+                        raise ValueError(f"{f.path}: sample identifiers differ from those of {ids_from}")
+            if sample_file is not None:
+                listed = _bgen.read_sample_file(sample_file)
+                if len(listed) != n:
+                    raise ValueError(f"{os.fspath(sample_file)} lists {len(listed)} samples, the BGEN files hold {n}")
+                if ids is not None and listed != ids:
+                    k = next(i for i, (a, b) in enumerate(zip(listed, ids)) if a != b)
+                    raise ValueError(f"{os.fspath(sample_file)}: sample {k} is {listed[k]!r}, {ids_from} embeds "
+                                     f"{ids[k]!r}")
+                ids, ids_from = listed, os.fspath(sample_file)
             p = sum(f.m for f in files)
             if n == 0 or p == 0:
                 raise _lib.DimensionMismatch(_lib.IHTB_EDIM, f"BGEN input must have n > 0 samples and p > 0 variants, "
                                                              f"got n = {n}, p = {p}")
-            variants = [v for f in files for v in f.variants]
-            jobs, j = [], 0
+            all_variants = [v for f in files for v in f.variants]
+            rows = _bgen_rows(samples, n, ids, ids_from)
+            cols = _bgen_cols(variants, all_variants)
+            if rows is not None and rows.shape[0] == 0:
+                raise _lib.DimensionMismatch(_lib.IHTB_EDIM, "the sample selection is empty")
+            if cols is not None and cols.shape[0] == 0:
+                raise _lib.DimensionMismatch(_lib.IHTB_EDIM, "the variant selection is empty")
+            kept_ids = ids if rows is None or ids is None else [ids[r] for r in rows.tolist()]
+            jobs, j, start = [], 0, 0
             for f in files:
-                for c0, c1 in f.batches(_bgen.INFLATE_BATCH_BYTES):
-                    jobs.append((f, c0, c1, j + c0))
-                j += f.m
-            return cls._load_bgen(jobs, n, p, variants, samples, standardize, allele, storage)
+                if cols is None:
+                    for c0, c1 in f.batches(_bgen.INFLATE_BATCH_BYTES):
+                        jobs.append((f, range(c0, c1), j + c0))
+                    j += f.m
+                else:
+                    lo, hi = np.searchsorted(cols, [start, start + f.m])
+                    for idx in f.variant_batches(cols[lo:hi] - start, _bgen.INFLATE_BATCH_BYTES):
+                        jobs.append((f, idx, j))
+                        j += idx.shape[0]
+                start += f.m
+            kept_variants = all_variants if cols is None else [all_variants[c] for c in cols.tolist()]
+            return cls._load_bgen(jobs, n, rows, kept_variants, kept_ids, standardize, allele, storage)
         finally:
             for f in files:
                 f.close()
 
     @classmethod
-    def _load_bgen(cls, jobs, n, p, variants, samples, standardize, allele, storage):
+    def _load_bgen(cls, jobs, n_file, rows, variants, samples, standardize, allele, storage):
         from . import bgen as _bgen
+        n = n_file if rows is None else rows.shape[0]
+        p = len(variants)
         lib = load()
         obj = None
         with ThreadPoolExecutor(max_workers=max(1, min(32, os.cpu_count() or 1))) as pool, \
                 ThreadPoolExecutor(max_workers=1) as ahead:
             def inflate(job):
-                f, c0, c1, _ = job
-                return f.inflate(c0, c1, pool)
+                f, idx, _ = job
+                return f.inflate(idx.start, idx.stop, pool) if isinstance(idx, range) else f.inflate_variants(idx, pool)
             nxt = ahead.submit(inflate, jobs[0])
             for t, job in enumerate(jobs):
                 buf, offs = nxt.result()
                 if t + 1 < len(jobs):
                     nxt = ahead.submit(inflate, jobs[t + 1])       # inflate the next batch while this one loads
-                f, c0, c1, jcol = job
-                bits = _bgen.block_bits(buf, offs, n)
+                f, idx, jcol = job
+                bits = _bgen.block_bits(buf, offs, n_file)
                 if obj is None:
                     b0 = int(bits[0])
                     if storage == "fix16" and not 1 <= b0 <= 15:
@@ -390,15 +429,17 @@ class B200DenseLinAlg:
                         check(lib.ihtb_geno_create_dense_empty(n, p, _lib.DENSE_F64, int(bool(standardize)), C.byref(h)))
                         obj = cls(h, n, p, np.float64, standardize)
                     obj.variants, obj.samples = variants, samples
+                    if rows is not None:
+                        check(lib.ihtb_geno_select_bgen_samples(obj._h, _lib.ptr(rows, C.c_int64), n_file))
                 if obj.denominator is not None:
                     other = np.flatnonzero(bits != b0)
                     if other.size:
-                        c = c0 + int(other[0])
+                        c = idx[int(other[0])]
                         raise ValueError(f"{f.path}: variant {f.variants[c].name()} stores B = {int(bits[other[0]])} "
                                          f"bits per probability, the first variant B = {b0}: 16-bit codes need one B "
                                          f"for all variants (use storage='f64')")
                 status = lib.ihtb_geno_load_bgen_columns(obj._h, _lib.ptr(buf, C.c_uint8), _lib.ptr(offs, C.c_int64),
-                                                         jcol, c1 - c0, int(allele))
+                                                         jcol, len(idx), int(allele))
                 if status != _lib.IHTB_OK:
                     raise _lib._EXC.get(status, _lib.IHTBError)(status, f"{f.path}: {_lib.last_error()}")
         check(lib.ihtb_geno_finalize(obj._h))
@@ -1056,6 +1097,78 @@ def _load_plink(filename: str, phenotypes, d: str):
     return x, y
 
 
+def _bgen_rows(samples, n: int, ids, ids_from):
+    """int64 file rows of from_bgen's `samples` (None: every sample in file order); ValueError names the first
+    unknown or repeated ID, out-of-range or repeated position, or IDs without an ID source."""
+    if samples is None:
+        return None
+    if isinstance(samples, (str, bytes)):
+        raise ValueError("samples must be a sequence of sample IDs or 0-based positions, not one string")
+    sel = list(samples)
+    if all(isinstance(s, str) for s in sel):
+        if sel and ids is None:
+            raise ValueError("samples lists IDs, but the BGEN files embed no sample IDs and no sample_file is given")
+        where = {}
+        twice = set()
+        for i, s in enumerate(ids or ()):
+            if s in where:
+                twice.add(s)
+            where.setdefault(s, i)
+        rows, seen = [], {}
+        for k, s in enumerate(sel):
+            if s not in where:
+                raise ValueError(f"samples[{k}] = {s!r} is not a sample ID of {ids_from}")
+            if s in twice:
+                raise ValueError(f"samples[{k}] = {s!r} names more than one sample of {ids_from}")
+            if s in seen:
+                raise ValueError(f"samples[{seen[s]}] and samples[{k}] are both {s!r}")
+            seen[s] = k
+            rows.append(where[s])
+        return np.asarray(rows, dtype=np.int64)
+    seen = {}
+    for k, s in enumerate(sel):
+        if isinstance(s, (bool, np.bool_)) or not isinstance(s, (int, np.integer)):
+            raise ValueError(f"samples[{k}] = {s!r}: samples must be all sample IDs (str) or all 0-based positions "
+                             f"(int)")
+        if not 0 <= s < n:
+            raise ValueError(f"samples[{k}] = {int(s)} is outside the file's samples [0, {n})")
+        if int(s) in seen:
+            raise ValueError(f"samples[{seen[int(s)]}] and samples[{k}] are both sample {int(s)}")
+        seen[int(s)] = k
+    return np.asarray([int(s) for s in sel], dtype=np.int64)
+
+
+def _bgen_cols(variants, all_variants):
+    """int64 kept columns of from_bgen's `variants` (None: every variant): a callable BgenVariant -> bool, a boolean
+    mask over the concatenated variants, or strictly increasing indices into them."""
+    p = len(all_variants)
+    if variants is None:
+        return None
+    if callable(variants):
+        return np.asarray([j for j, v in enumerate(all_variants) if variants(v)], dtype=np.int64)
+    sel = np.asarray(variants)
+    if sel.ndim != 1:
+        raise ValueError(f"variants must be one-dimensional, got shape {sel.shape}")
+    if sel.dtype == np.bool_:
+        if sel.shape[0] != p:
+            raise ValueError(f"the variant mask has {sel.shape[0]} entries, the files hold {p} variants")
+        return np.flatnonzero(sel).astype(np.int64)
+    if sel.shape[0] == 0:
+        return np.zeros(0, dtype=np.int64)
+    if not np.issubdtype(sel.dtype, np.integer):
+        raise ValueError(f"variants must be a boolean mask, integer indices or a callable, got {sel.dtype} entries")
+    bad = np.flatnonzero((sel < 0) | (sel >= p))
+    if bad.size:
+        k = int(bad[0])
+        raise ValueError(f"variants[{k}] = {int(sel[k])} is outside the files' variants [0, {p})")
+    down = np.flatnonzero(np.diff(sel) <= 0)
+    if down.size:
+        k = int(down[0]) + 1
+        raise ValueError(f"variants must be strictly increasing: variants[{k}] = {int(sel[k])} follows "
+                         f"{int(sel[k - 1])}")
+    return sel.astype(np.int64)
+
+
 def _bgen_input(filename: str):
     """The BGEN file that `filename` names (it ends in .bgen, or it is a prefix with prefix.bgen and no prefix.bed),
     else None: PLINK input keeps precedence."""
@@ -1067,11 +1180,17 @@ def _bgen_input(filename: str):
     return None
 
 
-def _load_input(filename: str, phenotypes, d: str):
+def _load_input(filename: str, phenotypes, d: str, samples=None, sample_file=None, variants=None):
     """(x, y) of PLINK or BGEN input.  BGEN dosages are standardized like the reference's dense dosages
-    (src/wrapper.jl:406-423); a BGEN file has no .fam, so phenotypes is an array or a comma-separated file."""
+    (src/wrapper.jl:406-423); a BGEN file has no .fam, so phenotypes is an array or a comma-separated file.  The BGEN
+    selection keywords go to from_bgen only when given."""
     path = _bgen_input(filename)
+    select = {k: v for k, v in (("samples", samples), ("sample_file", sample_file), ("variants", variants))
+              if v is not None}
     if path is None:
+        if select:
+            raise ValueError(f"{filename} is PLINK input: samples, sample_file and variants select from BGEN files "
+                             f"only (got {', '.join(select)})")
         return _load_plink(filename, phenotypes, d)
     if isinstance(phenotypes, (bool, int, np.integer)):
         raise ValueError(f"{path}: BGEN input has no .fam file to take phenotype column {phenotypes} from; pass "
@@ -1082,17 +1201,20 @@ def _load_input(filename: str, phenotypes, d: str):
         y = np.loadtxt(phenotypes, delimiter=",", dtype=np.float64)
         if y.ndim == 2:
             y = np.ascontiguousarray(y.T) if y.shape[1] > 1 else y[:, 0]
-    return B200DenseLinAlg.from_bgen(path, standardize=True), y
+    return B200DenseLinAlg.from_bgen(path, standardize=True, **select), y
 
 
 def iht(filename: str, k: int, d: str = NORMAL, phenotypes=6, covariates: str = "", summaryfile: str = None,
-        betafile: str = None, exclude_std_idx=(), **kwargs) -> IHTResult:
+        betafile: str = None, exclude_std_idx=(), samples=None, sample_file=None, variants=None,
+        **kwargs) -> IHTResult:
     """`iht(filename, k, d; phenotypes, covariates, ...)` (src/wrapper.jl:52-120) for binary PLINK input: reads
     `filename`.bed/.fam, builds the device genotype operator with center/scale/impute, standardises covariates and
     runs `fit_iht` with the canonical link (LogLink for NegativeBinomial).  Optional text outputs like the reference.
     BGEN input: `filename` ending in .bgen (or a prefix with prefix.bgen and no prefix.bed) is read with
-    `B200DenseLinAlg.from_bgen(standardize=True)`; `phenotypes` is then an array or a comma-separated file."""
-    x, y = _load_input(filename, phenotypes, d)
+    `B200DenseLinAlg.from_bgen(standardize=True)`; `phenotypes` is then an array or a comma-separated file, in the
+    row order of `samples`.  samples / sample_file / variants select BGEN samples and variants as in `from_bgen`; PLINK
+    input rejects them."""
+    x, y = _load_input(filename, phenotypes, d, samples, sample_file, variants)
     z = np.ones(x.n) if covariates == "" else parse_covariates(covariates, exclude_std_idx)
     if is_multivariate(y):          # src/wrapper.jl:80,84-85: z is transposed to q x n, no distribution / link
         z = np.ones((1, x.n)) if covariates == "" else np.ascontiguousarray(np.asarray(z).reshape(x.n, -1).T)
@@ -1113,9 +1235,11 @@ def iht(filename: str, k: int, d: str = NORMAL, phenotypes=6, covariates: str = 
 
 
 def cross_validate(filename: str, d: str = NORMAL, path=range(1, 21), q: int = 5, phenotypes=6, covariates: str = "",
-                   cv_summaryfile: str = None, exclude_std_idx=(), folds=None, **kwargs) -> np.ndarray:
-    """`cross_validate(filename, d; path, q, ...)` (src/wrapper.jl:301-349) for binary PLINK or BGEN input (as `iht`)."""
-    x, y = _load_input(filename, phenotypes, d)
+                   cv_summaryfile: str = None, exclude_std_idx=(), folds=None, samples=None, sample_file=None,
+                   variants=None, **kwargs) -> np.ndarray:
+    """`cross_validate(filename, d; path, q, ...)` (src/wrapper.jl:301-349) for binary PLINK or BGEN input (as `iht`,
+    with the same BGEN samples / sample_file / variants selection)."""
+    x, y = _load_input(filename, phenotypes, d, samples, sample_file, variants)
     z = np.ones(x.n) if covariates == "" else parse_covariates(covariates, exclude_std_idx)
     if is_multivariate(y):
         z = np.ones((1, x.n)) if covariates == "" else np.ascontiguousarray(np.asarray(z).reshape(x.n, -1).T)

@@ -150,19 +150,24 @@ class BgenFile:
     def inflate(self, c0: int, c1: int, pool: ThreadPoolExecutor = None):
         """(uint8 buffer, int64 offsets) of the inflated blocks of variants [c0, c1); zlib.decompress releases the GIL,
         so a thread pool inflates blocks in parallel.  Every block's N is checked against the header's."""
-        idx = range(c0, c1)
+        return self.inflate_variants(range(c0, c1), pool)
+
+    def inflate_variants(self, cols, pool: ThreadPoolExecutor = None):
+        """`inflate` over the variants `cols` (indices into `variants`, in the order given): only those blocks are
+        read and inflated."""
+        idx = [int(c) for c in cols]
         parts = list(pool.map(self._block, idx)) if pool is not None else [self._block(c) for c in idx]
         lens = np.fromiter((len(b) for b in parts), dtype=np.int64, count=len(parts))
         offsets = np.zeros(len(parts) + 1, dtype=np.int64)
         np.cumsum(lens, out=offsets[1:])
         buf = np.frombuffer(b"".join(parts), dtype=np.uint8) if parts else np.zeros(0, np.uint8)
-        for i, b in enumerate(parts):
+        for c, b in zip(idx, parts):
             if len(b) < 4:
-                raise ValueError(f"{self.path}: variant {c0 + i} ({self.variants[c0 + i].name()}): probability block "
+                raise ValueError(f"{self.path}: variant {c} ({self.variants[c].name()}): probability block "
                                  f"of {len(b)} bytes is truncated")
             (bn,) = struct.unpack_from("<I", b, 0)
             if bn != self.n:
-                raise ValueError(f"{self.path}: variant {c0 + i} ({self.variants[c0 + i].name()}) holds {bn} samples, "
+                raise ValueError(f"{self.path}: variant {c} ({self.variants[c].name()}) holds {bn} samples, "
                                  f"the header {self.n}")
         return buf, offsets
 
@@ -178,6 +183,20 @@ class BgenFile:
             out.append((c0, self.m))
         return out
 
+    def variant_batches(self, cols, target: int = INFLATE_BATCH_BYTES):
+        """`batches` over the strictly increasing variant indices `cols`: [int64 array of indices] of about `target`
+        inflated bytes each (at least one variant), so that a load inflates only the variants it keeps."""
+        cols = np.asarray(cols, dtype=np.int64)
+        out, k0, acc = [], 0, 0
+        for k, c in enumerate(cols.tolist()):
+            if k > k0 and acc + self.inflated_len[c] > target:
+                out.append(cols[k0:k])
+                k0, acc = k, 0
+            acc += int(self.inflated_len[c])
+        if cols.shape[0] > k0:
+            out.append(cols[k0:])
+        return out
+
     def close(self):
         if isinstance(self._mm, mmap.mmap):
             self._mm.close()
@@ -189,6 +208,31 @@ class BgenFile:
         self.close()
 
 
+def read_sample_file(path) -> list:
+    """The ID_1 column of an Oxford .sample file: line 1 holds the column names (the first is ID_1), line 2 the column
+    types (the first three are 0), then one whitespace-separated line per sample.  ID_1 is the identifier BGEN writers
+    embed.  Raises ValueError naming the line of a malformed header or a short line."""
+    path = os.fspath(path)
+    ids = []
+    with open(path, "r", encoding="utf-8") as f:
+        names = f.readline().split()
+        if not names or names[0] != "ID_1":
+            raise ValueError(f"{path}: line 1: the first column must be ID_1, got {' '.join(names)!r}")
+        types = f.readline().split()
+        if len(types) < 3 or types[:3] != ["0", "0", "0"]:
+            raise ValueError(f"{path}: line 2: the column types must start with 0 0 0, got {' '.join(types)!r}")
+        if len(types) != len(names):
+            raise ValueError(f"{path}: line 2: {len(types)} column types for {len(names)} columns")
+        for ln, line in enumerate(f, start=3):
+            fields = line.split()
+            if not fields:
+                continue
+            if len(fields) < len(names):
+                raise ValueError(f"{path}: line {ln}: {len(fields)} fields, the header names {len(names)} columns")
+            ids.append(fields[0])
+    return ids
+
+
 def block_bits(buf: np.ndarray, offsets: np.ndarray, n: int) -> np.ndarray:
     """B of every block of an inflated batch (0 where the block is too short to hold it)."""
     pos = offsets[:-1] + 9 + n
@@ -198,9 +242,10 @@ def block_bits(buf: np.ndarray, offsets: np.ndarray, n: int) -> np.ndarray:
     return out
 
 
-def decode_block(block: bytes, n: int, allele: int = 2):
+def decode_block(block: bytes, n: int, allele: int = 2, rows=None):
     """numpy twin of k_bgen_decode for one inflated block: (int64 codes[n], bool missing[n], B), code / (2^B - 1) the
-    dosage of `allele`.  Raises ValueError on everything the kernel rejects."""
+    dosage of `allele`.  Raises ValueError on everything the kernel rejects.  rows: the selected decode -- entry i is
+    file sample rows[i] (n is then the file's N), only kept samples are checked, and errors name file sample indices."""
     b = np.frombuffer(block, dtype=np.uint8)
     if b.shape[0] < 8:
         raise ValueError("block shorter than its header")
@@ -220,40 +265,45 @@ def decode_block(block: bytes, n: int, allele: int = 2):
     need = 10 + n + (2 * n * nbits + 7) // 8
     if b.shape[0] < need:
         raise ValueError("block shorter than its header + ceil(2 N B / 8) bytes")
+    idx = np.arange(n, dtype=np.int64) if rows is None else np.asarray(rows, dtype=np.int64)
+    who = "sample" if rows is None else "file sample"
+    ploidy = ploidy[idx]
     missing = (ploidy & 0x80) != 0
     bad = ~missing & ((ploidy & 63) != 2)
     if bad.any():
-        raise ValueError(f"sample {int(np.flatnonzero(bad)[0])} is not diploid (only diploid samples)")
+        raise ValueError(f"{who} {int(idx[bad].min())} is not diploid (only diploid samples)")
     bits = np.unpackbits(b[10 + n:need], bitorder="little")[:2 * n * nbits].reshape(2 * n, nbits).astype(np.uint64)
     vals = bits @ (np.uint64(1) << np.arange(nbits, dtype=np.uint64))
-    v0, v1 = vals[0::2].astype(np.int64), vals[1::2].astype(np.int64)
+    v0, v1 = vals[0::2].astype(np.int64)[idx], vals[1::2].astype(np.int64)[idx]
     den = (1 << nbits) - 1
     if phased:
         c2 = 2 * den - v0 - v1
     else:
         over = ~missing & (v0 + v1 > den)
         if over.any():
-            raise ValueError(f"sample {int(np.flatnonzero(over)[0])}: P(11) + P(12) exceeds 1 (a + b > 2^B - 1)")
+            raise ValueError(f"{who} {int(idx[over].min())}: P(11) + P(12) exceeds 1 (a + b > 2^B - 1)")
         c2 = v1 + 2 * (den - v0 - v1)
     codes = c2 if allele == 2 else 2 * den - c2
     codes = np.where(missing, 0, codes)
     return codes, missing, nbits
 
 
-def dosage_codes(path: str, allele: int = 2):
+def dosage_codes(path: str, allele: int = 2, rows=None, variants=None):
     """Host twin of the device ingest, for tests and small files: (int64 codes [n, p], bool missing [n, p], int64 B [p])
     with the dosage of `allele` (1 or 2) of sample i at variant j equal to codes[i, j] / (2^B[j] - 1); missing entries
-    have code 0."""
+    have code 0.  rows (file sample indices) and variants (variant indices) twin a selected load: row i is file sample
+    rows[i], column j is variant variants[j], and only those variants are inflated and decoded."""
     if allele not in (1, 2):
         raise ValueError(f"allele must be 1 or 2, got {allele!r}")
     with BgenFile(path) as f:
-        n, p = f.n, f.m
+        cols = range(f.m) if variants is None else [int(c) for c in variants]
+        n, p = (f.n if rows is None else len(rows)), len(cols)
         codes = np.zeros((n, p), dtype=np.int64)
         missing = np.zeros((n, p), dtype=bool)
         bits = np.zeros(p, dtype=np.int64)
-        for c in range(p):
+        for j, c in enumerate(cols):
             try:
-                codes[:, c], missing[:, c], bits[c] = decode_block(f._block(c), n, allele)
+                codes[:, j], missing[:, j], bits[j] = decode_block(f._block(c), f.n, allele, rows)
             except ValueError as e:
                 raise ValueError(f"{path}: variant {c} ({f.variants[c].name()}): {e}") from None
     return codes, missing, bits

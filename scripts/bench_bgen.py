@@ -12,7 +12,13 @@ then times each stage of B200DenseLinAlg.from_bgen separately in one process:
   end_to_end  from_bgen(path, standardize=True) as a user calls it (inflate overlapped with the device load)
 and the decode kernel's bytes/s (inflated bytes read + code bytes written) against a device-to-device copy in the same
 run (read + write bytes, torch, CUDA events, a buffer far larger than L2).  The card's name and power limit are read
-in the same run.  The loaded handle is checked against the host twin (bgen.dosage_codes) on its first variants."""
+in the same run.  The loaded handle is checked against the host twin (bgen.dosage_codes) on its first variants.
+
+Selection cases ("selection" in the output; from_bgen(samples=, variants=)), each timed the same way -- inflate of the
+kept variants, the decode kernel alone (torch.profiler), end-to-end from_bgen -- and checked against the host twin:
+  samples_50_sorted     every variant, half of the samples in file order
+  samples_50_shuffled   every variant, the same half in a random order (scattered reads inside each block)
+  variants_10           every sample, a random 10 % of the variants (the others are never inflated)"""
 import argparse
 import ctypes as C
 import json
@@ -79,6 +85,43 @@ def write_file(path: str, n: int, p: int, threads: int) -> None:
             meta = bw._s16(f"v{j}") + bw._s16(f"rs{j + 1}") + bw._s16("1") + struct.pack("<IH", 1000 + j, 2)
             meta += struct.pack("<I", 1) + b"A" + struct.pack("<I", 1) + b"G"
             f.write(meta + struct.pack("<II", len(z) + 4, len(blk)) + z)
+
+
+def selection_case(lib, path, f, rows, cols, threads):
+    """inflate / decode-kernel / end-to-end seconds of from_bgen(path, samples=rows, variants=cols)"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    n = f.n if rows is None else rows.shape[0]
+    out = {"n": n, "p": int(cols.shape[0])}
+    batches = f.variant_batches(cols)
+    out["inflated_bytes"] = int(f.inflated_len[cols].sum())
+    t0 = time.perf_counter()
+    with ThreadPoolExecutor(threads) as pool:
+        data = [f.inflate_variants(idx, pool) for idx in batches]
+    out["inflate_s"] = time.perf_counter() - t0
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        h = C.c_void_p()
+        _lib.check(lib.ihtb_geno_create_dosage16_empty(n, out["p"], 255, 1, C.byref(h)))
+        if rows is not None:
+            _lib.check(lib.ihtb_geno_select_bgen_samples(h, _lib.ptr(rows, C.c_int64), f.n))
+        j = 0
+        for idx, (buf, offs) in zip(batches, data):
+            _lib.check(lib.ihtb_geno_load_bgen_columns(h, _lib.ptr(buf, C.c_uint8), _lib.ptr(offs, C.c_int64), j,
+                                                       idx.shape[0], 2))
+            j += idx.shape[0]
+        torch.cuda.synchronize()
+    lib.ihtb_geno_destroy(h)
+    del data
+    out["decode_kernel_s"] = sum(ev.device_time for ev in prof.events() if "k_bgen_decode" in ev.name) / 1e6
+    t0 = time.perf_counter()
+    x = m.B200DenseLinAlg.from_bgen(path, standardize=True, samples=rows, variants=cols)
+    out["end_to_end_s"] = time.perf_counter() - t0
+    ref_cols = cols[:32]
+    codes, miss, _ = bgen.dosage_codes(path, rows=rows, variants=ref_cols)
+    ref = m.B200DenseLinAlg.from_array(np.asfortranarray(np.where(miss, np.nan, codes / 255.0)), standardize=True)
+    out["matches_twin"] = bool(np.array_equal(x.decode(0, n, 0, ref_cols.shape[0]).view(np.uint64),
+                                              ref.decode().view(np.uint64)))
+    return out
 
 
 def main():
@@ -167,6 +210,14 @@ def main():
         want = np.where(miss, np.nan, codes / 255.0)
         ref = m.B200DenseLinAlg.from_array(np.asfortranarray(want), standardize=True)
         res["matches_twin"] = bool(np.array_equal(x.decode(0, a.n, 0, 64).view(np.uint64), ref.decode().view(np.uint64)))
+        del x, ref
+        rng = np.random.default_rng(0)
+        half = np.sort(rng.choice(a.n, size=a.n // 2, replace=False))
+        every = np.arange(a.p, dtype=np.int64)
+        cases = {"samples_50_sorted": (half, every), "samples_50_shuffled": (rng.permutation(half), every),
+                 "variants_10": (None, np.sort(rng.choice(a.p, size=max(1, a.p // 10), replace=False)))}
+        res["selection"] = {name: selection_case(lib, path, f, rows, cols, a.threads)
+                            for name, (rows, cols) in cases.items()}
         f.close()
     stages = {k: res[k] for k in ("parse_s", "inflate_s", "load_s", "finalize_s")}
     res["slowest_stage"] = max(stages, key=stages.get)
